@@ -1,7 +1,8 @@
 #!/usr/bin/env python
-"""bench.py -- SMoE hot-path benchmark (contract in the task statement / DESIGN.md section "Measurement").
+"""bench.py -- SMoE hot-path benchmark (DESIGN.md section "Measurement").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c1|c2|c3|c4s|c4]
+                    [--dump-outputs DIR]
 
 One "step" = one full training iteration of the hot path on the workload: pi-mask compaction,
 fused forward (both sweeps), fused backward, statistics -> gradients, Adam, kernel-list upkeep.
@@ -322,6 +323,27 @@ def aux_hbm_pieces(m, img, peaks):
     return out
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(m, step_out, out_dir):
+    """Writes what the last timed step hands its caller as out_dir/<name>.npy: run_batched's loss, mse and active
+    kernel count (float64), the parameters after the step's Adam update, the step's gradients and the kernel
+    influence lists (float32).  The inputs are seeded, so two builds run with the same arguments can be compared
+    array by array."""
+    loss, mse, num_pi, _ = step_out
+    arrays = {"loss": np.float64([loss]), "mse": np.float64([mse]), "num_pi": np.float64([num_pi])}
+    arrays.update({f"params_{k}": np.asarray(v, np.float32) for k, v in m.get_params().items()})
+    arrays.update({f"grads_{k}": np.asarray(v, np.float32) for k, v in m.get_gradients().items()})
+    arrays["kernel_list"] = np.stack(m.kernel_list_per_batch).astype(np.float32)
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_ours(args):
     import torch
     import __graft_entry__ as ge
@@ -359,6 +381,8 @@ def run_ours(args):
             torch.distributed.barrier()
         torch.cuda.synchronize()
 
+    last_out = [None]           # run_batched's return value of the most recent timed step
+
     def timed_steps(mm, n, host_image=None, **kw):
         """n steps, each bracketed by its own CUDA events on the launching stream, L2 flushed
         (256 MB write) between steps outside the events; returns per-step ms (max over ranks)."""
@@ -370,7 +394,7 @@ def run_ours(args):
             e0.record()
             if host_image is not None:
                 mm.set_image(host_image)          # H2D of this step's pixels, inside the timed region
-            mm.run_batched(train=True, **kw)      # ends with the D2H read of the step's loss scalars + sync
+            last_out[0] = mm.run_batched(train=True, **kw)    # ends with the D2H read of the step's loss scalars + sync
             e1.record()
             torch.cuda.synchronize()
             t = torch.tensor([e0.elapsed_time(e1)], device="cuda")
@@ -392,6 +416,8 @@ def run_ours(args):
     n_timed_samples = len(sampler.rows) if rank == 0 else 0
     total_s = sum(ms) / 1e3
     value = evals_per_step * args.steps / total_s
+    if args.dump_outputs and rank == 0:
+        dump_outputs(m, last_out[0], args.dump_outputs)     # before the legs below move the model on
 
     # e2e: the same steps through the public API (Smoe.set_image + Smoe.run_batched) with this step's pixels coming
     # from pinned host memory -- the 8-bit pixels as an image file holds them; the /255 conversion (utils.py:126-128)
@@ -520,7 +546,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-dense", action="store_true", help="skip the dense_exec=1 roofline leg")
     ap.add_argument("--no-aux", action="store_true", help="skip the HBM-bound aux pieces")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -122,7 +122,7 @@ def test_sharded_ssim_region_scheme_equals_full_image(tmp_path):
     padding at the ring's borders) == SSIM sum of the whole image: a window centred within the block reaches at most 5
     pixels out, and the padding is only ever consulted at true image borders."""
     import torch.multiprocessing as mp
-    mp.spawn(_ssim_shard_worker, args=(2, 29611, str(tmp_path)), nprocs=2, join=True)
+    mp.spawn(_ssim_shard_worker, args=(2, _free_port(), str(tmp_path)), nprocs=2, join=True)
     part, full = np.load(os.path.join(str(tmp_path), "ssim.npy"))
     np.testing.assert_allclose(part, full, rtol=1e-12)
 
