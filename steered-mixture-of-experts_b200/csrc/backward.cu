@@ -190,6 +190,7 @@ __global__ void __launch_bounds__(kThreads, 512 / kThreads) backward_kernel(cons
     constexpr int T = tri(D);
     constexpr int P = nparam(D, C), PK = pstride(D, C);
     const int RL = a.b.tile[D - 1];          // pixels per row of the tile (run along the last axis)
+    const int NR = SMOE_TPIX / RL;           // rows per tile (a power of two: RL divides 128, smoe_forward checks it)
     const int tstride = pix_stride(D, C, RL);
     const uint32_t kTileBytes = (uint32_t)tstride * 4u;
     extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -231,27 +232,9 @@ __global__ void __launch_bounds__(kThreads, 512 / kThreads) backward_kernel(cons
         tma_load_1d(buf ? buf1 : buf0, a.pix + (size_t)tile * tstride, kTileBytes, &bar[buf]);
     };
 
-    // own kernel record (global -> registers)
-    float mu[D], Qm[D][D], c0, lam, kap[D], nu[C], ga[D][C];
-    {
-        const float* rec = a.packed + (size_t)(active ? k : 0) * PK;
-#pragma unroll
-        for (int l = 0; l < D; ++l) mu[l] = rec[off_mu(D, C) + l];
-#pragma unroll
-        for (int l = 0; l < D; ++l)
-#pragma unroll
-            for (int m = l; m < D; ++m) Qm[l][m] = Qm[m][l] = rec[off_A(D, C) + ut(D, l, m)];
-        c0 = active ? rec[off_pi(D, C)] : -INFINITY;
-        lam = rec[P];
-#pragma unroll
-        for (int l = 0; l < D; ++l) kap[l] = rec[P + 1 + l];
-#pragma unroll
-        for (int c = 0; c < C; ++c) nu[c] = rec[off_nu(D, C) + c];
-#pragma unroll
-        for (int l = 0; l < D; ++l)
-#pragma unroll
-            for (int c = 0; c < C; ++c) ga[l][c] = rec[off_ga(D, C) + l * C + c];
-    }
+    // own kernel record: read again at every tile (the CTA's kGroup records stay in L1) rather than held in registers
+    // across the tile loop -- the registers go to the look-ahead of the pixel loop below
+    const float* rec = a.packed + (size_t)(active ? k : 0) * PK;
 
     // ordered list of this split's tiles (s, s + NS, ...) that the group can reach, from the plan's bitmask
     int nlist = 0;
@@ -305,16 +288,18 @@ __global__ void __launch_bounds__(kThreads, 512 / kThreads) backward_kernel(cons
         tile_box_of<D>(a, tile, ctr, half);
         float mup[D];
 #pragma unroll
-        for (int l = 0; l < D; ++l) mup[l] = mu[l] - ctr[l];
+        for (int l = 0; l < D; ++l) mup[l] = __ldg(rec + off_mu(D, C) + l) - ctr[l];
+        const float c0 = active ? __ldg(rec + off_pi(D, C)) : -INFINITY;
         // own kernel vs this tile, then the warp's 32 kernels together
         bool need = active;
         if (cull && need) {
+            const float lam = __ldg(rec + P);
             float d2 = 0.f, kd = 0.f;
 #pragma unroll
             for (int l = 0; l < D; ++l) {
                 const float gap = fmaxf(fabsf(mup[l]) - half[l], 0.f);
                 d2 = fmaf(gap, gap, d2);
-                kd = fmaxf(kd, kap[l] * gap * gap);
+                kd = fmaxf(kd, __ldg(rec + P + 1 + l) * gap * gap);
             }
             const float ub = c0 - fmaxf(lam * d2, kd) - a.tile_qmin[tile];
             need = !(lam >= 0.f) || !(ub < zcut_tile);
@@ -326,6 +311,11 @@ __global__ void __launch_bounds__(kThreads, 512 / kThreads) backward_kernel(cons
             // tile-centred record in registers
             float f[R::RC];
             {
+                float Qm[D][D];
+#pragma unroll
+                for (int l = 0; l < D; ++l)
+#pragma unroll
+                    for (int m = l; m < D; ++m) Qm[l][m] = Qm[m][l] = __ldg(rec + off_A(D, C) + ut(D, l, m));
                 float v[D];
                 float qc = c0;
 #pragma unroll
@@ -345,11 +335,12 @@ __global__ void __launch_bounds__(kThreads, 512 / kThreads) backward_kernel(cons
                 f[R::OC] = qc;
 #pragma unroll
                 for (int c = 0; c < C; ++c) {
-                    float n = nu[c];
+                    float n = __ldg(rec + off_nu(D, C) + c);
 #pragma unroll
                     for (int l = 0; l < D; ++l) {
-                        n = fmaf(ga[l][c], ctr[l], n);
-                        f[R::OGA + l * C + c] = ga[l][c];
+                        const float g = __ldg(rec + off_ga(D, C) + l * C + c);
+                        n = fmaf(g, ctr[l], n);
+                        f[R::OGA + l * C + c] = g;
                     }
                     f[R::ONU + c] = n;
                 }
@@ -368,72 +359,111 @@ __global__ void __launch_bounds__(kThreads, 512 / kThreads) backward_kernel(cons
 
             // pixel state: planes [z | qthr | gr | g_c][512] + the row-constant coordinates (smoe_common.cuh)
             const float* pl = buf ? buf1 : buf0;
-            constexpr int GRP = 4;          // pixels tested together for the exact-zero skip
-            float s0 = 0.f, s1 = 0.f, s2 = 0.f, nv[C], nz[C];      // row sums, reset after every folded row
+            constexpr int GRP = 4;                               // pixels tested together for the exact-zero skip
+            constexpr int NGRP = SMOE_TPIX / (GRP * kHalves);    // groups a lane visits per tile: every kHalves-th row
+            const int gpr = RL / GRP;                            // groups per row
+            // the pixels of a row differ only in their LAST coordinate z: q = cr + (br + qz z) z
+            const float qz = f[R::OQ + ut(D, D - 1, D - 1)];
+            auto row_coords = [&](int row, float (&x)[3]) {
+                x[0] = x[1] = x[2] = 0.f;
 #pragma unroll
-            for (int c = 0; c < C; ++c) nv[c] = nz[c] = 0.f;
-            for (int r0 = hsel * RL; r0 < SMOE_TPIX; r0 += kHalves * RL) {
-                // the pixels of a row differ only in their LAST coordinate z: q = cr + (br + qq_last z) z
-                float xr[3] = {0.f, 0.f, 0.f};
-#pragma unroll
-                for (int l = 0; l < D - 1; ++l) xr[l] = pl[pix_rowc_offset(C) + l * (SMOE_TPIX / RL) + r0 / RL];
-                float cr = f[R::OC];
+                for (int l = 0; l < D - 1; ++l) x[l] = pl[pix_rowc_offset(C) + l * NR + row];
+            };
+            auto row_logit = [&](const float (&x)[3], float& cr, float& br) {
+                cr = f[R::OC];
 #pragma unroll
                 for (int l = 0; l < D - 1; ++l) {
                     float tq = f[R::OL + l];
 #pragma unroll
-                    for (int m = l; m < D - 1; ++m) tq = fmaf(f[R::OQ + ut(D, l, m)], xr[m], tq);
-                    cr = fmaf(tq, xr[l], cr);
+                    for (int m = l; m < D - 1; ++m) tq = fmaf(f[R::OQ + ut(D, l, m)], x[m], tq);
+                    cr = fmaf(tq, x[l], cr);
                 }
-                float br = f[R::OL + D - 1];
+                br = f[R::OL + D - 1];
 #pragma unroll
-                for (int l = 0; l < D - 1; ++l) br = fmaf(f[R::OQ + ut(D, l, D - 1)], xr[l], br);
-                const float qz = f[R::OQ + ut(D, D - 1, D - 1)];
-                // experts along the row: E_c = Er_c + gamma_{d-1,c} z
-                float Er[C];
+                for (int l = 0; l < D - 1; ++l) br = fmaf(f[R::OQ + ut(D, l, D - 1)], x[l], br);
+            };
+            // experts along the row: E_c = Er_c + gamma_{d-1,c} z
+            auto row_experts = [&](const float (&x)[3], float (&Er)[C]) {
 #pragma unroll
                 for (int c = 0; c < C; ++c) {
                     Er[c] = f[R::ONU + c];
 #pragma unroll
-                    for (int l = 0; l < D - 1; ++l) Er[c] = fmaf(f[R::OGA + l * C + c], xr[l], Er[c]);
+                    for (int l = 0; l < D - 1; ++l) Er[c] = fmaf(f[R::OGA + l * C + c], x[l], Er[c]);
                 }
-                // row sums: along a row only z varies, so sum t, sum t z, sum t z^2 (and sum v_c, sum v_c z)
-                // carry every moment of the row; they are folded once per row
-                bool row_active = false;
-                // (the two lanes of a kernel read rows RL floats apart, i.e. the same banks when RL = 32: a 2-way conflict
-                // on these broadcast loads; measured, walking the second row rotated by half a row costs more
-                // instructions than the conflicts cost LSU cycles -- the LSU pipe is at 16 %)
-                for (int j0 = r0; j0 < r0 + RL; j0 += GRP) {
-                    const float4 zv = *reinterpret_cast<const float4*>(pl + PL_Z * SMOE_TPIX + j0);
-                    const float4 tv = *reinterpret_cast<const float4*>(pl + PL_QTHR * SMOE_TPIX + j0);
-                    const float z4[GRP] = {zv.x, zv.y, zv.z, zv.w};
-                    const float t4[GRP] = {tv.x, tv.y, tv.z, tv.w};
-                    float dq[GRP];
-                    float dmax = -INFINITY;
+            };
+            // z, gr and the gate logits relative to the pixel's normaliser, dq = q - log2 S, of the group at pixel j
+            auto load_group = [&](int j, float cr, float br, float (&z)[GRP], float (&g)[GRP], float (&dq)[GRP]) {
+                const float4 zv = *reinterpret_cast<const float4*>(pl + PL_Z * SMOE_TPIX + j);
+                const float4 tv = *reinterpret_cast<const float4*>(pl + PL_QTHR * SMOE_TPIX + j);
+                const float4 gv = *reinterpret_cast<const float4*>(pl + PL_GR * SMOE_TPIX + j);
+                z[0] = zv.x; z[1] = zv.y; z[2] = zv.z; z[3] = zv.w;
+                g[0] = gv.x; g[1] = gv.y; g[2] = gv.z; g[3] = gv.w;
+                const float t[GRP] = {tv.x, tv.y, tv.z, tv.w};
 #pragma unroll
-                    for (int u = 0; u < GRP; ++u) {
-                        // gate logit relative to the pixel's normaliser: dq = q - log2 S
-                        dq[u] = fmaf(fmaf(qz, z4[u], br), z4[u], cr) - t4[u];
-                        dmax = fmaxf(dmax, dq[u]);
-                    }
-                    if (COUNT) cnt_vis += 1;
-                    // w = 2^dq is exactly +0 for dq < -126 (ex2.approx.ftz): nothing to accumulate
-                    if (__builtin_expect(skip && !__any_sync(0xffffffffu, dmax >= zcut), 1)) continue;
+                for (int u = 0; u < GRP; ++u) dq[u] = fmaf(fmaf(qz, z[u], br), z[u], cr) - t[u];
+            };
+
+            // Software pipeline over the lane's groups, across row boundaries: while group i is tested and
+            // accumulated, the loads and logits of group i+1 (in the next row, after the last group of a row) are
+            // already issued, so the two warp votes of a group never wait on a shared-memory round trip.
+            // (the row coordinates are read again where they are needed, instead of being held across the row)
+            int row = hsel;                                      // row of the look-ahead group
+            float cr, br, Er[C];
+            {
+                float x[3];
+                row_coords(row, x);
+                row_logit(x, cr, br);                            // (cr, br): row of the look-ahead group
+                row_experts(x, Er);
+            }
+            float zn[GRP], gn[GRP], dqn[GRP];                    // the look-ahead group
+            load_group(row * RL, cr, br, zn, gn, dqn);
+            int jn = row * RL, col = 0;
+            // row sums: along a row only z varies, so sum t, sum t z, sum t z^2 (and sum v_c, sum v_c z) carry every
+            // moment of the row; they are folded once per row and reset
+            float s0 = 0.f, s1 = 0.f, s2 = 0.f, nv[C], nz[C];
+#pragma unroll
+            for (int c = 0; c < C; ++c) nv[c] = nz[c] = 0.f;
+            bool row_active = false;
+            // (the two lanes of a kernel read rows RL floats apart, i.e. the same banks when RL = 32: a 2-way conflict
+            // on these broadcast loads; measured, walking the second row rotated by half a row costs more
+            // instructions than the conflicts cost LSU cycles -- the LSU pipe is at 16 %)
+            // (unrolled twice, so that the registers of the current and the look-ahead group alternate instead of
+            // being copied at every step)
+#pragma unroll 2
+            for (int gi = 0; gi < NGRP; ++gi) {
+                float z4[GRP], gr4[GRP], dq[GRP];
+#pragma unroll
+                for (int u = 0; u < GRP; ++u) { z4[u] = zn[u]; gr4[u] = gn[u]; dq[u] = dqn[u]; }
+                const int j0 = jn;
+                // look ahead: the next group of this row, or the first of the lane's next row (after the last row,
+                // the first row again -- loaded and never used)
+                const bool row_end = ++col == gpr;
+                const int rc = row;                              // the current row
+                if (row_end) {
+                    row = (row + kHalves) & (NR - 1);
+                    float x[3];
+                    row_coords(row, x);
+                    row_logit(x, cr, br);
+                    jn = row * RL;
+                } else {
+                    jn += GRP;
+                }
+                load_group(jn, cr, br, zn, gn, dqn);
+
+                // both warp decisions of the group, with no load between them:
+                //   some gate of the warp is nonzero -- w = 2^dq is exactly +0 for dq < -126 (ex2.approx.ftz);
+                //   some gate passes the threshold (w > tau) -- most groups with a nonzero gate only carry
+                //   sub-threshold ones: they need neither the g_c planes nor the expert part, only t = -w gr.
+                float dmax = -INFINITY;
+#pragma unroll
+                for (int u = 0; u < GRP; ++u) dmax = fmaxf(dmax, dq[u]);
+                const bool any_gate = !skip || __any_sync(0xffffffffu, dmax >= zcut);
+                const bool any_pass = !skip || __any_sync(0xffffffffu, dmax > ltau);
+                if (COUNT) cnt_vis += 1;
+                if (__builtin_expect(any_gate, 0)) {
                     if (COUNT) cnt_gate += 1;
                     row_active = true;
-                    const float4 grv = *reinterpret_cast<const float4*>(pl + PL_GR * SMOE_TPIX + j0);
-                    const float gr4[GRP] = {grv.x, grv.y, grv.z, grv.w};
-                    // does any gate of the group pass the threshold for any kernel of the warp?  Most groups that
-                    // reach this point only carry sub-threshold gates (w < tau): they need neither the g_c planes nor
-                    // the expert part, only t = -w gr and its moments.
-                    bool gpass = true;
-                    if (skip) {
-                        gpass = false;
-#pragma unroll
-                        for (int u = 0; u < GRP; ++u) gpass |= dq[u] > ltau;
-                        gpass = __any_sync(0xffffffffu, gpass);
-                    }
-                    if (!gpass) {
+                    if (!any_pass) {
 #pragma unroll
                         for (int u = 0; u < GRP; ++u) {
                             const float w = ex2f(dq[u]);             // e / S: the plane holds log2 S
@@ -443,22 +473,20 @@ __global__ void __launch_bounds__(kThreads, 512 / kThreads) backward_kernel(cons
                             s1 += uz;
                             s2 = fmaf(uz, z4[u], s2);
                         }
-                        continue;
-                    }
-                    float g4[C][GRP];
+                    } else {
+                        float g4[C][GRP];
 #pragma unroll
-                    for (int c = 0; c < C; ++c) {
-                        const float4 gv = *reinterpret_cast<const float4*>(pl + (PL_G + c) * SMOE_TPIX + j0);
-                        g4[c][0] = gv.x; g4[c][1] = gv.y; g4[c][2] = gv.z; g4[c][3] = gv.w;
-                    }
+                        for (int c = 0; c < C; ++c) {
+                            const float4 gv = *reinterpret_cast<const float4*>(pl + (PL_G + c) * SMOE_TPIX + j0);
+                            g4[c][0] = gv.x; g4[c][1] = gv.y; g4[c][2] = gv.z; g4[c][3] = gv.w;
+                        }
+                        // the expert part runs for all 4 pixels, with wm = 0 on those whose gate does not pass: adding
+                        // 0 * g is exact, so this is the dense instantiation's arithmetic, without a vote per pixel
+                        if (COUNT) cnt_exp += GRP;
 #pragma unroll
-                    for (int u = 0; u < GRP; ++u) {
-                        const float w = ex2f(dq[u]);                 // e / S: the plane holds log2 S
-                        float t = -w * gr4[u];
-                        const bool pass = dq[u] > ltau;              // w > tau
-                        if (!skip || __any_sync(0xffffffffu, pass)) {
-                            if (COUNT) cnt_exp += 1;
-                            const float wm = pass ? w : 0.f;
+                        for (int u = 0; u < GRP; ++u) {
+                            const float w = ex2f(dq[u]);             // e / S: the plane holds log2 S
+                            const float wm = dq[u] > ltau ? w : 0.f; // w > tau
                             float gE = 0.f;
 #pragma unroll
                             for (int c = 0; c < C; ++c) {
@@ -468,36 +496,44 @@ __global__ void __launch_bounds__(kThreads, 512 / kThreads) backward_kernel(cons
                                 nv[c] += vc;
                                 nz[c] = fmaf(vc, z4[u], nz[c]);
                             }
-                            t = fmaf(wm, gE, t);
+                            const float t = fmaf(wm, gE, -w * gr4[u]);
+                            const float uz = t * z4[u];
+                            s0 += t;
+                            s1 += uz;
+                            s2 = fmaf(uz, z4[u], s2);
                         }
-                        const float uz = t * z4[u];
-                        s0 += t;
-                        s1 += uz;
-                        s2 = fmaf(uz, z4[u], s2);
                     }
                 }
-                if (row_active) {
-                    // fold the row: x_l = xr[l] for l < D-1, x_{D-1} = z
-                    M0 += s0;
+                if (row_end) {
+                    float xr[3];
+                    if (row_active) {
+                        // fold the row: x_l = xr[l] for l < D-1, x_{D-1} = z
+                        row_coords(rc, xr);
+                        M0 += s0;
 #pragma unroll
-                    for (int l = 0; l < D - 1; ++l) {
-                        const float a0 = xr[l] * s0;
-                        M1[l] += a0;
+                        for (int l = 0; l < D - 1; ++l) {
+                            const float a0 = xr[l] * s0;
+                            M1[l] += a0;
 #pragma unroll
-                        for (int m = l; m < D - 1; ++m) M2[ut(D, l, m)] = fmaf(a0, xr[m], M2[ut(D, l, m)]);
-                        M2[ut(D, l, D - 1)] = fmaf(xr[l], s1, M2[ut(D, l, D - 1)]);
+                            for (int m = l; m < D - 1; ++m) M2[ut(D, l, m)] = fmaf(a0, xr[m], M2[ut(D, l, m)]);
+                            M2[ut(D, l, D - 1)] = fmaf(xr[l], s1, M2[ut(D, l, D - 1)]);
+                        }
+                        M1[D - 1] += s1;
+                        M2[ut(D, D - 1, D - 1)] += s2;
+#pragma unroll
+                        for (int c = 0; c < C; ++c) {
+                            N0[c] += nv[c];
+#pragma unroll
+                            for (int l = 0; l < D - 1; ++l) N1[l][c] = fmaf(xr[l], nv[c], N1[l][c]);
+                            N1[D - 1][c] += nz[c];
+                            nv[c] = nz[c] = 0.f;
+                        }
+                        s0 = s1 = s2 = 0.f;
+                        row_active = false;
                     }
-                    M1[D - 1] += s1;
-                    M2[ut(D, D - 1, D - 1)] += s2;
-#pragma unroll
-                    for (int c = 0; c < C; ++c) {
-                        N0[c] += nv[c];
-#pragma unroll
-                        for (int l = 0; l < D - 1; ++l) N1[l][c] = fmaf(xr[l], nv[c], N1[l][c]);
-                        N1[D - 1][c] += nz[c];
-                        nv[c] = nz[c] = 0.f;
-                    }
-                    s0 = s1 = s2 = 0.f;
+                    row_coords(row, xr);
+                    row_experts(xr, Er);
+                    col = 0;
                 }
             }
             // fold tile-centred statistics into kernel-centred ones
