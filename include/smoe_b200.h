@@ -46,8 +46,9 @@
 extern "C" {
 #endif
 
-#define SMOE_ABI_VERSION 3   /* 3: Hilbert-ordered packing (perm argument of smoe_pack, influence flags by ORIGINAL index,
-                                smoe_backward without perm/pos), executed-pair counters, eps_bits, peer exchange */
+#define SMOE_ABI_VERSION 4   /* 3: Hilbert-ordered packing (perm argument of smoe_pack, influence flags by ORIGINAL index,
+                                smoe_backward without perm/pos), executed-pair counters, eps_bits, peer exchange;
+                                4: smoe_cotangent added (additive: every call of version 3 is unchanged) */
 #define SMOE_TPIX 512      /* pixels per tile (compile-time constant of the kernels) */
 #define SMOE_NSCAL 16      /* floats in the scalar block */
 
@@ -211,6 +212,16 @@ int smoe_loss_partials(const smoe_batch* batch);
 int smoe_loss(const smoe_cfg* cfg, const smoe_batch* batch, const float* rbuf, const float* image,
               const uint8_t* image_u8, const float* loss_weights, float* res, float* pix, float* scalars,
               float* partials, int32_t* ticket, void* stream);
+
+/* Any upstream gradient into the backward state, in place of smoe_loss, after smoe_forward (with pix) and before
+ * smoe_backward: the loss is the caller's (a PyTorch loss, a larger network), the library only needs its dL/dr.
+ *   grad_r   [dims..][C]  dL/dr with r the mixture output BEFORE clip (the rbuf of smoe_forward), same layout as rbuf
+ *   pix      the forward's state: per pixel slot of every tile, g_c = grad_r (0 outside the batch rectangle) and
+ *            gr = sum_c g_c r_c (fmaf in channel order from 0, as smoe_loss) where S > 1e-11, else 0 (smoe.py:821)
+ * One CTA per tile, the launch geometry of smoe_loss; elementwise, HBM-bound, no reduction, no atomics.  The batch has
+ * no halo.  The flag "S > 1e-11" that smoe_forward leaves is consumed: call it once per smoe_forward. */
+int smoe_cotangent(const smoe_cfg* cfg, const smoe_batch* batch, const float* rbuf, const float* grad_r, float* pix,
+                   void* stream);
 
 /* Fused backward over one batch: recomputes the gates from the per-pixel state and reduces the
  * per-kernel sufficient statistics (sum t, sum t*delta, sum t*delta*delta^T, sum m*w*g,

@@ -14,13 +14,13 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libsmoe_b200.so")
 
 TPIX = 512
-ABI_VERSION = 3           # SMOE_ABI_VERSION of include/smoe_b200.h
+ABI_VERSION = 4           # SMOE_ABI_VERSION of include/smoe_b200.h (4 adds smoe_cotangent; version 3 calls unchanged)
 NSCAL = 16
 STATS_STRIDE = 24         # floats per batch in the host-visible block: scalars | counts | regsums | pad (16-byte rows)
 
 EXPORTS = [
     "smoe_abi_version", "smoe_last_error", "smoe_param_count", "smoe_packed_stride", "smoe_num_tiles", "smoe_pix_stride",
-    "smoe_pack_workspace_bytes", "smoe_backward_workspace_bytes", "smoe_backward_plan_bytes", "smoe_pack", "smoe_pack_fed", "smoe_forward", "smoe_loss", "smoe_loss_partials", "smoe_ssim_loss_workspace_bytes", "smoe_ssim_loss",
+    "smoe_pack_workspace_bytes", "smoe_backward_workspace_bytes", "smoe_backward_plan_bytes", "smoe_pack", "smoe_pack_fed", "smoe_forward", "smoe_loss", "smoe_loss_partials", "smoe_cotangent", "smoe_ssim_loss_workspace_bytes", "smoe_ssim_loss",
     "smoe_backward", "smoe_suggest_splits", "smoe_reduce_splits", "smoe_grad_finalize", "smoe_update_kernel_list",
     "smoe_adam_step", "smoe_step_begin", "smoe_spatial_keys", "smoe_xchg_window_bytes", "smoe_peer_alloc", "smoe_peer_free",
     "smoe_peer_export", "smoe_peer_open", "smoe_peer_close", "smoe_xchg_publish", "smoe_grad_finalize_peers",

@@ -2,6 +2,7 @@
 // smoe.py:899-937, 1053.  The forward needs no target pixels: it leaves the mixture output r (before clip) and the
 // gate state; smoe_loss then clips, fake-quantises, compares with the target and writes dL/dr for the backward.
 // Keeping the two apart lets a step's target arrive from the host WHILE the sweeps run (the end-to-end path).
+// smoe_cotangent is the other way into the backward: it writes a caller's dL/dr instead of the library's loss.
 //
 // Pixel-stationary: a CTA (128 threads, 6 resident per SM for images, 4 for video) owns a spatially compact tile of
 // SMOE_TPIX = 512 pixels (4 per thread, in registers) and streams the active kernels past it twice:
@@ -687,6 +688,62 @@ __global__ void __launch_bounds__(256) loss_kernel(const LossArgs a) {
     }
 }
 
+// ---- cotangent stage --------------------------------------------------------------------------------------
+// The alternative to loss_kernel before the backward when the loss lives outside the library: an arbitrary dL/dr
+// (grad_r, same layout as rbuf) goes into the g_c / gr planes of the pixel state.  Same launch geometry and slot
+// numbering as loss_kernel, and the same arithmetic for gr (fmaf over the channels in order, from 0), so a grad_r
+// equal to what loss_kernel derives yields the same planes bit for bit.  Elementwise, HBM-bound: reads grad_r and r
+// (C floats each) and the "S > 1e-11" flag, writes 1 + C plane values per pixel.  No reduction, no atomics.
+struct CotArgs {
+    smoe_batch b;
+    const float* rbuf;
+    const float* grad_r;
+    float* pix;
+    int nt1, nt2, pix_tstride;
+};
+
+template <int C>
+__global__ void __launch_bounds__(256) cotangent_kernel(const CotArgs a) {
+    const int tid = threadIdx.x;
+    const int e1 = a.b.tile[1], e2 = a.b.tile[2];
+    int tt[3], lo[3], hi[3];
+    tt[0] = blockIdx.y;
+    tt[1] = a.nt2 == 1 ? (int)blockIdx.x : (int)blockIdx.x / a.nt2;
+    tt[2] = a.nt2 == 1 ? 0 : (int)blockIdx.x % a.nt2;
+    const int tile = (tt[0] * a.nt1 + tt[1]) * a.nt2 + tt[2];
+#pragma unroll
+    for (int i = 0; i < 3; ++i) {
+        lo[i] = a.b.origin[i] + tt[i] * a.b.tile[i];
+        hi[i] = min(lo[i] + a.b.tile[i], a.b.origin[i] + a.b.extent[i]) - 1;
+    }
+    float* tp = a.pix + (size_t)tile * a.pix_tstride;
+    const int i2 = tid % e2, i1 = (tid / e2) % e1;
+    const int g1 = lo[1] + i1, g2 = lo[2] + i2;
+    const bool in12 = g1 <= hi[1] && g2 <= hi[2];
+    const int rows_per_pass = 256 / (e1 * e2);
+    int g0 = lo[0] + tid / (e1 * e2);
+    for (int j = tid; j < SMOE_TPIX; j += 256, g0 += rows_per_pass) {
+        const bool inb = in12 && g0 <= hi[0];
+        const int gpix = inb ? (g0 * a.b.dims[1] + g1) * a.b.dims[2] + g2 : 0;
+        float g[C], gr = 0.f;
+#pragma unroll
+        for (int c = 0; c < C; ++c) g[c] = 0.f;
+        if (inb) {
+#pragma unroll
+            for (int c = 0; c < C; ++c) {
+                const size_t gi = (size_t)gpix * C + c;
+                g[c] = a.grad_r[gi];
+                gr = fmaf(g[c], a.rbuf[gi], gr);
+            }
+        }
+        // g_c reaches the gate gradients of a clamped pixel too; gr only where S > 1e-11 (smoe.py:821)
+        const bool live = tp[PL_GR * SMOE_TPIX + j] != 0.f;
+        tp[PL_GR * SMOE_TPIX + j] = live ? gr : 0.f;
+#pragma unroll
+        for (int c = 0; c < C; ++c) tp[(PL_G + c) * SMOE_TPIX + j] = g[c];
+    }
+}
+
 template <int D, int C>
 static size_t fwd_smem_bytes(int max_chunks) {
     return (size_t)(2 * kChunk * pstride(D, C) + kChunk * Rec<D, C>::RC) * 4 + 2 * 8 + 32 * 4 + 8 * 4 +
@@ -785,4 +842,25 @@ extern "C" int smoe_loss(const smoe_cfg* cfg, const smoe_batch* batch, const flo
     if (cfg->C == 1) loss_kernel<1><<<grid, 256, 0, (cudaStream_t)stream>>>(a);
     else loss_kernel<3><<<grid, 256, 0, (cudaStream_t)stream>>>(a);
     return check_launch("smoe_loss");
+}
+
+extern "C" int smoe_cotangent(const smoe_cfg* cfg, const smoe_batch* batch, const float* rbuf, const float* grad_r,
+                              float* pix, void* stream) {
+    SMOE_REQUIRE(cfg && batch && rbuf && grad_r && pix, "null argument");
+    SMOE_REQUIRE(batch->tile[0] * batch->tile[1] * batch->tile[2] == SMOE_TPIX, "tile product must be SMOE_TPIX");
+    SMOE_REQUIRE(batch->halo == 0, "halo must be 0: the cotangent covers the whole batch rectangle");
+    SMOE_REQUIRE((cfg->d == 2 || cfg->d == 3) && (cfg->C == 1 || cfg->C == 3), "d in {2, 3} and 1 or 3 channels");
+    SMOE_REQUIRE(256 % (batch->tile[1] * batch->tile[2]) == 0, "tile[1]*tile[2] must divide 256");
+    CotArgs a;
+    a.b = *batch;
+    a.rbuf = rbuf; a.grad_r = grad_r; a.pix = pix;
+    a.nt1 = (batch->extent[1] + batch->tile[1] - 1) / batch->tile[1];
+    a.nt2 = (batch->extent[2] + batch->tile[2] - 1) / batch->tile[2];
+    a.pix_tstride = pix_stride(cfg->d, cfg->C, batch->tile[cfg->d - 1]);
+    const int nt0 = smoe_num_tiles(batch) / (a.nt1 * a.nt2);
+    SMOE_REQUIRE(nt0 <= 65535, "too many tiles along the first axis");
+    const dim3 grid(a.nt1 * a.nt2, nt0);
+    if (cfg->C == 1) cotangent_kernel<1><<<grid, 256, 0, (cudaStream_t)stream>>>(a);
+    else cotangent_kernel<3><<<grid, 256, 0, (cudaStream_t)stream>>>(a);
+    return check_launch("smoe_cotangent");
 }

@@ -37,6 +37,40 @@ from .quantizer import quantize_params, rescaler
 PARAM_KEYS = ("pis", "musX", "A_diagonal", "A_corr", "gamma_e", "nu_e")
 
 
+def theta_offsets(d, C):
+    """First column of each variable in a theta row (include/smoe_b200.h): musX | A lower triangle | pis | nu_e |
+    gamma_e."""
+    T = d * (d + 1) // 2
+    return dict(mu=0, A=d, pi=d + T, nu=d + T + 1, ga=d + T + 1 + C)
+
+
+def a_col(d, l, m):
+    """Column of A[l, m] (l >= m) in a theta row: the lower triangle, row-major."""
+    return d + l * (l + 1) // 2 + m
+
+
+def choose_tile(d, n_last):
+    """Tile extents (product SMOE_TPIX) of a batch of dimension d whose last axis has n_last samples."""
+    if d == 2:
+        return (_ffi.TPIX // 32, 32, 1)
+    # tile[1]*tile[2] must divide 128 and tile[2] must be a multiple of 4 (include/smoe_b200.h)
+    t2 = 8 if n_last > 4 else 4
+    t1 = 64 // t2
+    return (_ffi.TPIX // (t1 * t2), t1, t2)
+
+
+def key_scale(shape):
+    """Per-axis scale of the Hilbert keys (smoe_spatial_keys): n_a / max n, so the curve is isotropic in pixels."""
+    nmax = float(max(shape))
+    return (C.c_float * 3)(*([n / nmax for n in shape] + [1.0] * (3 - len(shape))))
+
+
+def backward_splits(k_eff, batches):
+    """Pixel splits of smoe_backward for k_eff kernels with work (at least 64) over `batches`; SMOE_SPLITS overrides."""
+    return int(os.environ.get("SMOE_SPLITS", 0)) or max(int(lib().smoe_suggest_splits(max(64, k_eff), C.byref(b)))
+                                                        for b in batches)
+
+
 def sliding_window(image, Overlap, BatchSize):
     """Yields (coord, window) over the domain axes, first axis outermost, last innermost, with a
     zero halo of `Overlap` (smoe.py:18-35)."""
@@ -379,7 +413,7 @@ class Smoe:
         self._P = L.smoe_param_count(d, Cc)
         self._PK = L.smoe_packed_stride(d, Cc)
         self._T = d * (d + 1) // 2
-        self._off = dict(mu=0, A=d, pi=d + self._T, nu=d + self._T + 1, ga=d + self._T + 1 + Cc)
+        self._off = theta_offsets(d, Cc)
         lb3 = float(self.lower_bounds[3]) if self.quantize_pis else 0.0
         ub3 = float(self.upper_bounds[3]) if self.quantize_pis else 1.0
         bits3 = int(self.bit_depths[3]) if self.quantize_pis else 8
@@ -408,11 +442,11 @@ class Smoe:
         if self.radial_as:          # one scalar per kernel on every diagonal entry, A_corr frozen at 0 (smoe.py:429-434)
             a0 = A0 if A0.ndim == 1 else A0[:, 0, 0]
             for l in range(d):
-                theta[:, d + l * (l + 1) // 2 + l] = a0
+                theta[:, a_col(d, l, l)] = a0
         else:
             for l in range(d):
                 for m in range(l + 1):
-                    theta[:, d + l * (l + 1) // 2 + m] = A0[:, l, m]
+                    theta[:, a_col(d, l, m)] = A0[:, l, m]
         theta[:, self._off["pi"]] = self.pis_init
         theta[:, self._off["nu"]:self._off["nu"] + Cc] = self.nu_e_init
         theta[:, self._off["ga"]:] = np.asarray(self.gamma_e_init).reshape(K, d * Cc)
@@ -461,7 +495,7 @@ class Smoe:
         self._d_res_pre = torch.zeros((npx, Cc), dtype=f32, device=dev)      # mixture output before clip (the forward's rbuf)
         self._d_argmax = torch.zeros((npx,), dtype=torch.int32, device=dev)
         # batches (smoe.py:1643: sliding_window order, first axis outermost)
-        self._tile = self._choose_tile()
+        self._tile = choose_tile(d, self._local_shape[d - 1])
         self._batches = []
         if self._world > 1:
             rects = [(tuple(sl.start for sl in self._blk_in_buf), self._local_shape)]
@@ -514,8 +548,7 @@ class Smoe:
         self._pos = torch.zeros((K,), dtype=torch.int32, device=dev)
         self._perm = torch.zeros((K,), dtype=torch.int32, device=dev)
         self._keys = torch.zeros((K,), dtype=torch.int64, device=dev)
-        nmax = float(max(self.image.shape[:d]))
-        self._key_scale = (C.c_float * 3)(*([self.image.shape[a] / nmax for a in range(d)] + [1.0] * (3 - d)))
+        self._key_scale = key_scale(self.image.shape[:d])
         self._refresh_perm()
         # one block per batch [scalars (NSCAL) | counts (4 x int32) | regulariser sums (2) | pad]: a single
         # device->host copy per run_batched call brings back everything the host needs
@@ -541,9 +574,7 @@ class Smoe:
         reach = self._reach_px()
         frac = float(np.prod([min(1.0, (self._local_shape[a] + 2 * reach[a]) / (self.image.shape[a] + 2 * reach[a]))
                               for a in range(d)]))
-        k_eff = max(64, int(K * frac))
-        self._splits = int(os.environ.get("SMOE_SPLITS", 0)) or max(int(L.smoe_suggest_splits(k_eff, C.byref(b)))
-                                                                    for b in self._batches)
+        self._splits = backward_splits(int(K * frac), self._batches)
         self._plan = torch.zeros((max(L.smoe_backward_plan_bytes(K, C.byref(b)) for b in self._batches) + 3) // 4,
                                  dtype=torch.int32, device=dev)
         self._raw_part = None           # allocated on the first training pass
@@ -705,16 +736,6 @@ class Smoe:
         self._enable_res_pre()
         self.run_batched(train=False, update_reconstruction=True)
         return self._d_res_pre.reshape(self._buf_shape + (self.image.shape[-1],))[self._blk_in_buf].cpu().numpy()
-
-    def _choose_tile(self):
-        d = self.dim_domain
-        if d == 2:
-            return (_ffi.TPIX // 32, 32, 1)
-        # tile[1]*tile[2] must divide 128 and tile[2] must be a multiple of 4 (include/smoe_b200.h)
-        T = self._local_shape[2]
-        t2 = 8 if T > 4 else 4
-        t1 = 64 // t2
-        return (_ffi.TPIX // (t1 * t2), t1, t2)
 
     # kernel_list_per_batch is exposed as the reference's list of NumPy bool arrays
     @property
@@ -1291,7 +1312,7 @@ class Smoe:
         th = self._effective_theta()
         for l in range(d):
             for m in range(l + 1):
-                A[:, l, m] = th[:, d + l * (l + 1) // 2 + m]
+                A[:, l, m] = th[:, a_col(d, l, m)]
                 if self.train_inverse_cov and m < l:
                     A[:, m, l] = A[:, l, m]
         return A
@@ -1352,7 +1373,7 @@ class Smoe:
             A_diag[:], A_corr[:] = sv[0], sv[1]
         for l in range(d):
             for m in range(l + 1):
-                (A_diag if l == m else A_corr)[:, l, m] = th[:, d + l * (l + 1) // 2 + m]
+                (A_diag if l == m else A_corr)[:, l, m] = th[:, a_col(d, l, m)]
         if self.radial_as:                                     # the (K,) variable (smoe.py:429-433)
             A_diag = th[:, d].copy()
         return {"pis": pis, "musX": th[:, 0:d].copy(), "A_diagonal": A_diag, "A_corr": A_corr,
@@ -1377,9 +1398,9 @@ class Smoe:
                 if key in params and self.radial_as:
                     if l == m:
                         a = np.asarray(params[key])
-                        th[:, d + l * (l + 1) // 2 + m] = a if a.ndim == 1 else a[:, 0, 0]
+                        th[:, a_col(d, l, m)] = a if a.ndim == 1 else a[:, 0, 0]
                 elif key in params:
-                    th[:, d + l * (l + 1) // 2 + m] = np.asarray(params[key])[:, l, m]
+                    th[:, a_col(d, l, m)] = np.asarray(params[key])[:, l, m]
         if "pis" in params:
             th[:, o["pi"]] = params["pis"]
         if "nu_e" in params:
@@ -1400,7 +1421,7 @@ class Smoe:
         A_corr = np.zeros((K, d, d), dtype=np.float32)
         for l in range(d):
             for m in range(l + 1):
-                (A_diag if l == m else A_corr)[:, l, m] = g[:, d + l * (l + 1) // 2 + m]
+                (A_diag if l == m else A_corr)[:, l, m] = g[:, a_col(d, l, m)]
         if self.radial_as:                  # gradient of the one scalar per kernel (every diagonal entry carries it)
             A_diag = g[:, d].copy()
         return {"pis": g[:, o["pi"]].copy(), "musX": g[:, 0:d].copy(), "A_diagonal": A_diag, "A_corr": A_corr,
