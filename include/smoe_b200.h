@@ -46,9 +46,10 @@
 extern "C" {
 #endif
 
-#define SMOE_ABI_VERSION 4   /* 3: Hilbert-ordered packing (perm argument of smoe_pack, influence flags by ORIGINAL index,
+#define SMOE_ABI_VERSION 5   /* 3: Hilbert-ordered packing (perm argument of smoe_pack, influence flags by ORIGINAL index,
                                 smoe_backward without perm/pos), executed-pair counters, eps_bits, peer exchange;
-                                4: smoe_cotangent added (additive: every call of version 3 is unchanged) */
+                                4: smoe_cotangent added (additive: every call of version 3 is unchanged);
+                                5: the smoe_point_* calls added (additive: every call of version 4 is unchanged) */
 #define SMOE_TPIX 512      /* pixels per tile (compile-time constant of the kernels) */
 #define SMOE_NSCAL 16      /* floats in the scalar block */
 
@@ -241,6 +242,40 @@ size_t smoe_backward_plan_bytes(int K_cap, const smoe_batch* batch);
 /* number of pixel splits for smoe_backward on this batch (split s owns tiles s, s+NS, ...): a prime that keeps
  * the grid a few waves deep and does not divide the tile-grid extents */
 int smoe_suggest_splits(int K_cap, const smoe_batch* batch);
+
+/* ---- evaluation at arbitrary points (csrc/points.cu) ------------------------------------------------------------
+ * The model at n_points coordinates points[n][d] instead of on a uniform grid, differentiable in the parameters and in
+ * the coordinates.  The points arrive in TILE ORDER: a point tile is a run of SMOE_TPIX consecutive points (the last
+ * one may be partial), and culling works on each tile's bounding box, so any order is correct and a spatially coherent
+ * one (e.g. sorted along a Hilbert curve with smoe_spatial_keys) is fast.  Coordinates must be finite; a tile with a
+ * NaN coordinate culls nothing.  cfg->eps_bits must be 0; cfg->dense_exec 0, 1 and 2 give the same bits.
+ *   smoe_point_forward    r[n][C] (before clip) at every point, from the smoe_pack records (chunk bounds included).
+ *                         With state != NULL (then tile_box too) also the backward state, per tile of
+ *                         smoe_point_stride floats: planes qthr | gr | g_c | tile-centred x'_l of SMOE_TPIX floats,
+ *                         and tile_box[tiles][8] = centre[3] | rounded-out half extent[3] | min qthr | 0
+ *   smoe_point_cotangent  a caller's dL/dr ([n][C], point order of r) into the state: g_c, and gr = sum_c g_c r_c where
+ *                         S > 1e-11, else 0; call it once per smoe_point_forward, before the two calls below
+ *   smoe_point_backward   planning pre-pass (every group of 32 packed kernels against every tile box) + kernel-
+ *                         stationary sweep into raw_part [num_splits][K_cap][P] and `plan` (smoe_point_plan_bytes), the
+ *                         layouts of smoe_backward: smoe_grad_finalize turns them into parameter gradients
+ *   smoe_point_xgrad      grad_points[n][d] = dL/dx per point (pixel-stationary, fixed kernel order, no atomics)
+ * smoe_point_splits gives num_splits from K_cap and n_points alone. */
+#define SMOE_POINT_MAX 2147483136   /* 2^31 - 512: largest n_points */
+int    smoe_point_tiles(int n_points);
+int    smoe_point_stride(int d, int C);      /* floats of `state` per tile */
+size_t smoe_point_plan_bytes(int K_cap, int n_points);
+int    smoe_point_splits(int K_cap, int n_points);
+int smoe_point_forward(const smoe_cfg* cfg, const float* packed, const int32_t* counts, const float* chunk_bounds,
+                       int K_cap, const float* points, int n_points, float* r, float* state /*or NULL*/,
+                       float* tile_box /*[tiles][8] with state*/, void* stream);
+int smoe_point_cotangent(const smoe_cfg* cfg, int n_points, const float* r, const float* grad_r, float* state,
+                         void* stream);
+int smoe_point_backward(const smoe_cfg* cfg, const float* packed, const int32_t* counts, int K_cap, int n_points,
+                        const float* state, const float* tile_box, int num_splits, float* raw_part, int32_t* plan,
+                        void* stream);
+int smoe_point_xgrad(const smoe_cfg* cfg, const float* packed, const int32_t* counts, const float* chunk_bounds,
+                     int K_cap, int n_points, const float* state, const float* tile_box, float* grad_points,
+                     void* stream);
 
 /* Fixed-order reduction of the pixel splits: raw[k][j] = sum_s raw_part[s][k][j].  (The buffer a
  * multi-GPU run all-reduces with NCCL.) */

@@ -14,4 +14,4 @@ from .smoe import Smoe, AdamOptimizer, sliding_window  # noqa: E402,F401
 from .quantizer import quantize_params, rescaler        # noqa: E402,F401
 from .utils import reduce_params, save_model, load_params, read_image, write_image, psnr  # noqa: E402,F401
 from . import smoe_reconstruction, smoe_reconstruction_decoded, smoe_test  # noqa: E402,F401
-from .render import SmoeRenderer  # noqa: E402,F401
+from .render import SmoePointRenderer, SmoeRenderer  # noqa: E402,F401

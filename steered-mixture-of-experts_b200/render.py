@@ -1,4 +1,5 @@
-"""`SmoeRenderer`: a differentiable SMoE render for PyTorch on any uniform grid.
+"""`SmoeRenderer` and `SmoePointRenderer`: differentiable SMoE evaluation for PyTorch, on any uniform grid and at any
+set of points.
 
 The training path (`Smoe.run_batched`) samples the model on the pixel grid of its own image and back-propagates its
 own loss.  An SMoE is a continuous function, so a user may want it on another grid -- a finer one
@@ -13,9 +14,10 @@ stage replaced by smoe_cotangent, which writes whatever dL/dr autograd hands bac
     loss.backward()          # gradients in params[k].grad, the reference's variable layout
 
 Each axis is `(start, stop, n)`: `np.linspace(start, stop, n)` cast to float32, as the training path builds its
-coordinates, so `(0, 1, n)` reproduces them bit for bit.  Grids that are not uniform cannot be expressed: the
-backward's tile planner relies on uniform spacing.  Gates, the threshold tau = 0.5 / 2^precision (no
-renormalisation), the determinant, `train_inverse_cov` and the exact culling are the training path's own kernels.
+coordinates, so `(0, 1, n)` reproduces them bit for bit.  Grids that are not uniform, and any other set of
+coordinates, go to `SmoePointRenderer` (below), which also differentiates in the coordinates.  Gates, the threshold
+tau = 0.5 / 2^precision (no renormalisation), the determinant, `train_inverse_cov` and the exact culling are the
+training path's own kernels.
 Fake quantisation, radial A, `use_diff_center` and kernel lists are not part of the op; a caller applies them in
 torch to the tensors it passes.  Nothing synchronises with the host, so the op can be captured in a CUDA graph.
 """
@@ -101,6 +103,80 @@ def check_params(params, d, C):
     return tuple(params[k] for k in PARAM_KEYS)
 
 
+def check_options(precision, dense_exec):
+    if isinstance(precision, bool) or not isinstance(precision, (int, np.integer)) or not 1 <= precision <= 30:
+        raise ValueError("precision must be an integer in [1, 30]")
+    if dense_exec not in (0, 1, 2):
+        raise ValueError("_dense_exec must be 0, 1 or 2")
+
+
+def resolve_device(device, who):
+    _ffi.require_cuda()
+    dev = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
+    if dev.type != "cuda":
+        raise ValueError(f"{who} runs on a CUDA device")
+    return torch.device("cuda", torch.cuda.current_device()) if dev.index is None else dev
+
+
+def make_cfg(d, C_, precision, use_determinant, train_inverse_cov, dense_exec):
+    """The training path's configuration of a model without quantisation; the loss fields (margin, use_yuv) are not
+    read by the calls the renderers make."""
+    return Cfg(d=d, C=C_, precision=int(precision), use_determinant=int(bool(use_determinant)),
+               train_inverse_cov=int(bool(train_inverse_cov)), train_gammas=1, pis_lb=0.0, pis_ub=1.0, pis_bits=8,
+               q_ub=(C.c_float * 5)(*[1.0] * 5), q_bits=(C.c_int32 * 5)(*[8] * 5), dense_exec=int(dense_exec))
+
+
+def pack_model(cfg, ts, scale):
+    """The six parameter tensors -> theta rows, Hilbert keys of the centres (smoe_spatial_keys, per-axis `scale`), a
+    stable sort and smoe_pack on the current stream.  Returns (theta, packed, indices, counts, chunk_bounds)."""
+    L, st, f32, i32 = lib(), stream_ptr(), torch.float32, torch.int32
+    d, Cc = cfg.d, cfg.C
+    P, PK = L.smoe_param_count(d, Cc), L.smoe_packed_stride(d, Cc)
+    pis, musX, A_diag, A_corr, gamma_e, nu_e = (t.detach() for t in ts)
+    dev = pis.device
+    K = pis.shape[0]
+    A_cols = torch.stack([A_diag[:, l, l] if l == m else A_corr[:, l, m] for l in range(d) for m in range(l + 1)], 1)
+    theta = torch.cat([musX, A_cols, pis[:, None], nu_e, gamma_e.reshape(K, d * Cc)], 1).contiguous()
+    keys = torch.empty((K,), dtype=torch.int64, device=dev)
+    check(L.smoe_spatial_keys(ptr(theta), K, d, P, ptr(None), scale, ptr(keys), st), "smoe_spatial_keys")
+    perm = torch.sort(keys, stable=True).indices.to(i32)
+    kernel_list = torch.ones((K,), dtype=torch.uint8, device=dev)
+    packed = torch.empty((K, PK), dtype=f32, device=dev)
+    indices = torch.empty((K,), dtype=i32, device=dev)
+    pos = torch.empty((K,), dtype=i32, device=dev)
+    counts = torch.empty((4,), dtype=i32, device=dev)
+    regsums = torch.empty((2,), dtype=f32, device=dev)
+    chunk_bounds = torch.empty(((K + 127) // 128, 12), dtype=f32, device=dev)
+    ws = torch.empty(((L.smoe_pack_workspace_bytes(K) + 15) // 4,), dtype=i32, device=dev)
+    check(L.smoe_pack(C.byref(cfg), ptr(theta), ptr(None), ptr(None), ptr(kernel_list), ptr(perm), K,
+                      ptr(packed), ptr(indices), ptr(pos), ptr(counts), ptr(regsums), ptr(chunk_bounds), ptr(ws),
+                      ptr(None), ptr(None), ptr(None), st), "smoe_pack")
+    return theta, packed, indices, counts, chunk_bounds
+
+
+def finalize_grads(cfg, raw_part, splits, plan, theta, indices, counts):
+    """smoe_grad_finalize of a backward's statistics without regularisers -> the (K, P) gradient rows of theta."""
+    K, P = theta.shape
+    grads = torch.zeros((K, P), dtype=torch.float32, device=theta.device)
+    check(lib().smoe_grad_finalize(C.byref(cfg), ptr(raw_part), splits, ptr(plan), K, ptr(theta), ptr(None),
+                                   ptr(indices), ptr(counts), C.c_float(0.0), C.c_float(float(K)), C.c_float(0.0),
+                                   ptr(grads), stream_ptr()), "smoe_grad_finalize")
+    return grads
+
+
+def split_grads(grads, d, Cc):
+    """(K, P) gradient rows -> the params-dict layout, in PARAM_KEYS order."""
+    o = theta_offsets(d, Cc)
+    K = grads.shape[0]
+    gA = torch.zeros((K, d, d), dtype=grads.dtype, device=grads.device)
+    gC = torch.zeros_like(gA)
+    for l in range(d):
+        for m in range(l + 1):
+            (gA if l == m else gC)[:, l, m] = grads[:, a_col(d, l, m)]
+    return (grads[:, o["pi"]].contiguous(), grads[:, 0:d].contiguous(), gA, gC,
+            grads[:, o["ga"]:].reshape(K, d, Cc).contiguous(), grads[:, o["nu"]:o["nu"] + Cc].contiguous())
+
+
 class SmoeRenderer:
     """Differentiable render of an SMoE on a uniform grid; see the module docstring.
 
@@ -119,29 +195,14 @@ class SmoeRenderer:
     def __init__(self, grid, channels=3, use_determinant=False, train_inverse_cov=False, precision=8, device=None,
                  _dense_exec=0):
         axes, _, batch = plan_grid(grid, channels)
-        if isinstance(precision, bool) or not isinstance(precision, (int, np.integer)) or not 1 <= precision <= 30:
-            raise ValueError("precision must be an integer in [1, 30]")
-        if _dense_exec not in (0, 1, 2):
-            raise ValueError("_dense_exec must be 0, 1 or 2")
-        _ffi.require_cuda()
+        check_options(precision, _dense_exec)
+        self.device = resolve_device(device, "SmoeRenderer")
         L = lib()
-        self.device = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
-        if self.device.type != "cuda":
-            raise ValueError("SmoeRenderer runs on a CUDA device")
-        if self.device.index is None:
-            self.device = torch.device("cuda", torch.cuda.current_device())
         d = len(axes)
         self.d, self.C = d, int(channels)
         self.shape = tuple(len(x) for x in axes)
         self._batch = batch
-        # the training path's configuration of a model without quantisation; the loss fields (margin, use_yuv) are
-        # not read by the calls this op makes
-        self._cfg = Cfg(d=d, C=self.C, precision=int(precision), use_determinant=int(bool(use_determinant)),
-                        train_inverse_cov=int(bool(train_inverse_cov)), train_gammas=1, pis_lb=0.0, pis_ub=1.0,
-                        pis_bits=8, q_ub=(C.c_float * 5)(*[1.0] * 5), q_bits=(C.c_int32 * 5)(*[8] * 5),
-                        dense_exec=int(_dense_exec))
-        self._P, self._PK = L.smoe_param_count(d, self.C), L.smoe_packed_stride(d, self.C)
-        self._off = theta_offsets(d, self.C)
+        self._cfg = make_cfg(d, self.C, precision, use_determinant, train_inverse_cov, _dense_exec)
         self._key_scale = key_scale(self.shape)
         self._ntiles = L.smoe_num_tiles(C.byref(batch))
         self._pix_floats = self._ntiles * L.smoe_pix_stride(d, self.C, C.byref(batch))
@@ -163,26 +224,10 @@ class SmoeRenderer:
     def _forward(self, ts, keep_state):
         """smoe_spatial_keys + sort + smoe_pack + smoe_forward on the current stream; with keep_state also the
         per-pixel state the backward needs."""
-        L, st, dev, f32, i32 = lib(), stream_ptr(), self.device, torch.float32, torch.int32
-        d, Cc, P, PK = self.d, self.C, self._P, self._PK
-        pis, musX, A_diag, A_corr, gamma_e, nu_e = (t.detach() for t in ts)
-        K = pis.shape[0]
-        A_cols = torch.stack([A_diag[:, l, l] if l == m else A_corr[:, l, m] for l in range(d) for m in range(l + 1)], 1)
-        theta = torch.cat([musX, A_cols, pis[:, None], nu_e, gamma_e.reshape(K, d * Cc)], 1).contiguous()
-        keys = torch.empty((K,), dtype=torch.int64, device=dev)
-        check(L.smoe_spatial_keys(ptr(theta), K, d, P, ptr(None), self._key_scale, ptr(keys), st), "smoe_spatial_keys")
-        perm = torch.sort(keys, stable=True).indices.to(i32)
-        kernel_list = torch.ones((K,), dtype=torch.uint8, device=dev)
-        packed = torch.empty((K, PK), dtype=f32, device=dev)
-        indices = torch.empty((K,), dtype=i32, device=dev)
-        pos = torch.empty((K,), dtype=i32, device=dev)
-        counts = torch.empty((4,), dtype=i32, device=dev)
-        regsums = torch.empty((2,), dtype=f32, device=dev)
-        chunk_bounds = torch.empty(((K + 127) // 128, 12), dtype=f32, device=dev)
-        ws = torch.empty(((L.smoe_pack_workspace_bytes(K) + 15) // 4,), dtype=i32, device=dev)
-        check(L.smoe_pack(C.byref(self._cfg), ptr(theta), ptr(None), ptr(None), ptr(kernel_list), ptr(perm), K,
-                          ptr(packed), ptr(indices), ptr(pos), ptr(counts), ptr(regsums), ptr(chunk_bounds), ptr(ws),
-                          ptr(None), ptr(None), ptr(None), st), "smoe_pack")
+        L, st, dev, f32 = lib(), stream_ptr(), self.device, torch.float32
+        Cc = self.C
+        theta, packed, indices, counts, chunk_bounds = pack_model(self._cfg, ts, self._key_scale)
+        K = theta.shape[0]
         out = torch.empty(self.shape + (Cc,), dtype=f32, device=dev)
         pix = torch.empty((self._pix_floats,), dtype=f32, device=dev) if keep_state else None
         tile_qmin = torch.empty((self._ntiles,), dtype=f32, device=dev) if keep_state else None
@@ -205,23 +250,7 @@ class SmoeRenderer:
         check(L.smoe_backward(C.byref(self._cfg), C.byref(self._batch), ptr(packed), ptr(counts), K, ptr(pix),
                               ptr(tile_qmin), *self._axis_ptrs(), splits, ptr(raw_part), ptr(plan), ptr(None), st),
               "smoe_backward")
-        grads = torch.zeros((K, P), dtype=torch.float32, device=dev)
-        check(L.smoe_grad_finalize(C.byref(self._cfg), ptr(raw_part), splits, ptr(plan), K, ptr(theta), ptr(None),
-                                   ptr(indices), ptr(counts), C.c_float(0.0), C.c_float(float(K)), C.c_float(0.0),
-                                   ptr(grads), st), "smoe_grad_finalize")
-        return grads
-
-    def _split_grads(self, grads):
-        """(K, P) gradient rows -> the params-dict layout, in PARAM_KEYS order."""
-        d, Cc, o = self.d, self.C, self._off
-        K = grads.shape[0]
-        gA = torch.zeros((K, d, d), dtype=grads.dtype, device=grads.device)
-        gC = torch.zeros_like(gA)
-        for l in range(d):
-            for m in range(l + 1):
-                (gA if l == m else gC)[:, l, m] = grads[:, a_col(d, l, m)]
-        return (grads[:, o["pi"]].contiguous(), grads[:, 0:d].contiguous(), gA, gC,
-                grads[:, o["ga"]:].reshape(K, d, Cc).contiguous(), grads[:, o["nu"]:o["nu"] + Cc].contiguous())
+        return finalize_grads(self._cfg, raw_part, splits, plan, theta, indices, counts)
 
 
 class _Render(torch.autograd.Function):
@@ -245,5 +274,152 @@ class _Render(torch.autograd.Function):
         with torch.cuda.device(r.device):
             grads = r._backward(out, ctx.state, grad_out.to(torch.float32).contiguous())
             ctx.state = None
-            parts = r._split_grads(grads)
+            parts = split_grads(grads, r.d, r.C)
         return (None,) + tuple(g if need else None for g, need in zip(parts, ctx.needs_input_grad[1:]))
+
+
+MAX_POINTS = 2147483136        # SMOE_POINT_MAX: point indices of the tiles stay below 2^31
+
+
+def check_points(points, d, device):
+    """The points tensor (..., d) -> its row count N; raises ValueError for a type, dtype, device or shape mismatch,
+    N = 0 and N > MAX_POINTS."""
+    if not isinstance(points, torch.Tensor):
+        raise ValueError(f"points must be a torch.Tensor, got {type(points).__name__}")
+    if points.dtype != torch.float32:
+        raise ValueError(f"points must be float32, got {points.dtype}")
+    if points.device != device:
+        raise ValueError(f"points are on {points.device}, the renderer on {device}")
+    if points.dim() < 1 or points.shape[-1] != d:
+        raise ValueError(f"points must have shape (..., {d}), got {tuple(points.shape)}")
+    n = points.numel() // d
+    if n < 1:
+        raise ValueError("points must hold at least one point")
+    if n > MAX_POINTS:
+        raise ValueError(f"{n} points; at most {MAX_POINTS} are supported")
+    return n
+
+
+class SmoePointRenderer:
+    """Differentiable evaluation of an SMoE at arbitrary points, in the parameters and in the coordinates.
+
+    d         2 (image) or 3 (video)
+    channels  1 or 3
+    use_determinant, train_inverse_cov, precision: as the `Smoe` constructor
+    device    the CUDA device of the params and points (default: the current one)
+
+    `r(params, points)` takes the params dict of `SmoeRenderer` and a float32 CUDA tensor of coordinates (..., d) and
+    returns the mixture r before clip at every point, (..., C), in the caller's order.  Gradients reach the params as
+    with `SmoeRenderer`, and `points` when it requires grad: dL/dx through the gates, the normaliser and the experts
+    (the 0/1 gate decision w > tau is a step, whose derivative is 0 almost everywhere).
+
+    Internally the points are sorted along a Hilbert curve over their bounding box (smoe_spatial_keys, a stable sort)
+    and gathered into tiles of 512; outputs and point gradients are scattered back.  The order only affects speed,
+    never the result.  Coordinates must be finite: a NaN or infinite coordinate is the caller's responsibility (that
+    point's values are undefined, and its tile of 512 points is evaluated without culling).  Nothing synchronises with the host.  Under
+    no_grad no backward state is allocated; in the backward, the parameter sweep runs only when a parameter needs a
+    gradient and the coordinate sweep only when the points do.  A call's backward runs once."""
+
+    def __init__(self, d=2, channels=3, use_determinant=False, train_inverse_cov=False, precision=8, device=None,
+                 _dense_exec=0):
+        if isinstance(d, bool) or d not in (2, 3):
+            raise ValueError("d must be 2 (image) or 3 (video)")
+        if isinstance(channels, bool) or channels not in (1, 3):
+            raise ValueError("channels must be 1 or 3")
+        check_options(precision, _dense_exec)
+        self.device = resolve_device(device, "SmoePointRenderer")
+        self.d, self.C = int(d), int(channels)
+        self._cfg = make_cfg(self.d, self.C, precision, use_determinant, train_inverse_cov, _dense_exec)
+        self._stride = lib().smoe_point_stride(self.d, self.C)
+        self._key_scale = key_scale((1,) * self.d)         # model coordinates: one scale on every axis
+
+    def __call__(self, params, points):
+        ts = check_params(params, self.d, self.C)
+        for k, t in zip(PARAM_KEYS, ts):
+            if t.device != self.device:
+                raise ValueError(f"params[{k!r}] is on {t.device}, the renderer on {self.device}")
+        check_points(points, self.d, self.device)
+        if torch.is_grad_enabled() and (points.requires_grad or any(t.requires_grad for t in ts)):
+            return _PointRender.apply(self, points, *ts)
+        with torch.cuda.device(self.device):
+            return self._forward(points, ts, keep_state=False)[0]
+
+    def _order(self, pts):
+        """Stable Hilbert order of the points over their bounding box (one scale for every axis), on the device."""
+        lo = pts.amin(0)
+        ext = (pts.amax(0) - lo).amax()
+        unit = (pts - lo) * torch.where(ext > 0, 1.0 / ext, torch.ones_like(ext))
+        keys = torch.empty((pts.shape[0],), dtype=torch.int64, device=pts.device)
+        check(lib().smoe_spatial_keys(ptr(unit.contiguous()), pts.shape[0], self.d, self.d, ptr(None), ptr(None),
+                                      ptr(keys), stream_ptr()), "smoe_spatial_keys")
+        return torch.sort(keys.to(torch.int32), stable=True).indices       # d * 10 bits: half the radix passes
+
+    def _forward(self, points, ts, keep_state):
+        """pack_model + point ordering + smoe_point_forward on the current stream; with keep_state also the point state
+        the backward needs."""
+        L, st, dev, f32 = lib(), stream_ptr(), self.device, torch.float32
+        pts = points.detach().reshape(-1, self.d)
+        n = pts.shape[0]
+        theta, packed, indices, counts, chunk_bounds = pack_model(self._cfg, ts, self._key_scale)
+        K = theta.shape[0]
+        order = self._order(pts)
+        sp = pts.index_select(0, order).contiguous()
+        r = torch.empty((n, self.C), dtype=f32, device=dev)
+        ntiles = L.smoe_point_tiles(n)
+        state = torch.empty((ntiles * self._stride,), dtype=f32, device=dev) if keep_state else None
+        tile_box = torch.empty((ntiles, 8), dtype=f32, device=dev) if keep_state else None
+        check(L.smoe_point_forward(C.byref(self._cfg), ptr(packed), ptr(counts), ptr(chunk_bounds), K, ptr(sp), n,
+                                   ptr(r), ptr(state), ptr(tile_box), st), "smoe_point_forward")
+        out = torch.empty_like(r).index_copy_(0, order, r)
+        return out.reshape(points.shape[:-1] + (self.C,)), (theta, packed, indices, counts, chunk_bounds, order, r,
+                                                           state, tile_box)
+
+    def _backward(self, state, grad_out, need_params, need_points):
+        """smoe_point_cotangent, then smoe_point_backward + smoe_grad_finalize (need_params) and smoe_point_xgrad
+        (need_points); returns the (K, P) gradient rows of theta or None, and dL/dx (N, d) or None."""
+        L, st, dev, f32 = lib(), stream_ptr(), self.device, torch.float32
+        theta, packed, indices, counts, chunk_bounds, order, r, pstate, tile_box = state
+        K, P = theta.shape
+        n = r.shape[0]
+        g = grad_out.reshape(-1, self.C).index_select(0, order).contiguous()
+        check(L.smoe_point_cotangent(C.byref(self._cfg), n, ptr(r), ptr(g), ptr(pstate), st), "smoe_point_cotangent")
+        grads = gx = None
+        if need_params:
+            splits = L.smoe_point_splits(K, n)
+            raw_part = torch.empty((splits * K * P,), dtype=f32, device=dev)
+            plan = torch.empty(((L.smoe_point_plan_bytes(K, n) + 3) // 4,), dtype=torch.int32, device=dev)
+            check(L.smoe_point_backward(C.byref(self._cfg), ptr(packed), ptr(counts), K, n, ptr(pstate), ptr(tile_box),
+                                        splits, ptr(raw_part), ptr(plan), st), "smoe_point_backward")
+            grads = finalize_grads(self._cfg, raw_part, splits, plan, theta, indices, counts)
+        if need_points:
+            gs = torch.empty((n, self.d), dtype=f32, device=dev)
+            check(L.smoe_point_xgrad(C.byref(self._cfg), ptr(packed), ptr(counts), ptr(chunk_bounds), K, n, ptr(pstate),
+                                     ptr(tile_box), ptr(gs), st), "smoe_point_xgrad")
+            gx = torch.empty_like(gs).index_copy_(0, order, gs)
+        return grads, gx
+
+
+class _PointRender(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, renderer, points, *ts):
+        with torch.cuda.device(renderer.device):
+            out, state = renderer._forward(points, ts, keep_state=True)
+        ctx.renderer = renderer
+        ctx.state = state
+        ctx.points_shape = points.shape
+        return out
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad_out):
+        if ctx.state is None:
+            raise RuntimeError("SmoePointRenderer: a call's backward runs once (smoe_point_cotangent consumes the "
+                               "forward's point state); evaluate again for another backward pass")
+        r = ctx.renderer
+        need_points, need_params = ctx.needs_input_grad[1], any(ctx.needs_input_grad[2:])
+        with torch.cuda.device(r.device):
+            grads, gx = r._backward(ctx.state, grad_out.to(torch.float32).contiguous(), need_params, need_points)
+            ctx.state = None
+            parts = split_grads(grads, r.d, r.C) if grads is not None else (None,) * len(PARAM_KEYS)
+        return ((None, gx.reshape(ctx.points_shape) if gx is not None else None)
+                + tuple(g if need else None for g, need in zip(parts, ctx.needs_input_grad[2:])))
