@@ -46,10 +46,12 @@
 extern "C" {
 #endif
 
-#define SMOE_ABI_VERSION 5   /* 3: Hilbert-ordered packing (perm argument of smoe_pack, influence flags by ORIGINAL index,
+#define SMOE_ABI_VERSION 6   /* 3: Hilbert-ordered packing (perm argument of smoe_pack, influence flags by ORIGINAL index,
                                 smoe_backward without perm/pos), executed-pair counters, eps_bits, peer exchange;
                                 4: smoe_cotangent added (additive: every call of version 3 is unchanged);
-                                5: the smoe_point_* calls added (additive: every call of version 4 is unchanged) */
+                                5: the smoe_point_* calls added (additive: every call of version 4 is unchanged);
+                                6: smoe_point_jacobian and smoe_jacobian added (additive: every call of version 5 is
+                                   unchanged) */
 #define SMOE_TPIX 512      /* pixels per tile (compile-time constant of the kernels) */
 #define SMOE_NSCAL 16      /* floats in the scalar block */
 
@@ -276,6 +278,23 @@ int smoe_point_backward(const smoe_cfg* cfg, const float* packed, const int32_t*
 int smoe_point_xgrad(const smoe_cfg* cfg, const float* packed, const int32_t* counts, const float* chunk_bounds,
                      int K_cap, int n_points, const float* state, const float* tile_box, float* grad_points,
                      void* stream);
+
+/* ---- spatial Jacobian at arbitrary points and on a grid (csrc/jacobian.cu) -----------------------------------------
+ * jac[n][C][d] = d r_c / d x_l at every point (tile order), the derivative of r before clip, from the state and
+ * tile_box of a smoe_point_forward call with state and its r ([n][C], tile order).  Call it before
+ * smoe_point_cotangent, which overwrites the flag S > 1e-11 the forward leaves in the gr plane.  One pixel-stationary
+ * sweep: every kernel above the exact-zero cut, in packed order, no float atomics; as for dL/dx, the 0/1 gate decision
+ * w > tau contributes no term.  cfg->eps_bits must be 0; cfg->dense_exec 0, 1 and 2 give the same bits. */
+int smoe_point_jacobian(const smoe_cfg* cfg, const float* packed, const int32_t* counts, const float* chunk_bounds,
+                        int K_cap, int n_points, const float* state, const float* tile_box, const float* r, float* jac,
+                        void* stream);
+/* The same Jacobian on a uniform grid: jac[pixel][C][d] in rbuf's layout, per unit of the axes' coordinate, from the
+ * pix and tile_qmin of a smoe_forward call on `batch` (which must have halo 0) and its rbuf; the tile geometry and
+ * coordinates are recomputed from the batch and the axes as the forward computes them.  Call it before smoe_loss or
+ * smoe_cotangent, which overwrite the flag in the gr plane. */
+int smoe_jacobian(const smoe_cfg* cfg, const smoe_batch* batch, const float* packed, const int32_t* counts,
+                  const float* chunk_bounds, int K_cap, const float* pix, const float* tile_qmin, const float* ax0,
+                  const float* ax1, const float* ax2 /*NULL when d == 2*/, const float* rbuf, float* jac, void* stream);
 
 /* Fixed-order reduction of the pixel splits: raw[k][j] = sum_s raw_part[s][k][j].  (The buffer a
  * multi-GPU run all-reduces with NCCL.) */

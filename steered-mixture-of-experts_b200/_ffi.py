@@ -14,7 +14,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libsmoe_b200.so")
 
 TPIX = 512
-ABI_VERSION = 5           # SMOE_ABI_VERSION of include/smoe_b200.h (5 adds the smoe_point_* calls; version 4 calls unchanged)
+ABI_VERSION = 6           # SMOE_ABI_VERSION of include/smoe_b200.h (6 adds smoe_point_jacobian, smoe_jacobian; v5 calls unchanged)
 NSCAL = 16
 STATS_STRIDE = 24         # floats per batch in the host-visible block: scalars | counts | regsums | pad (16-byte rows)
 
@@ -26,7 +26,8 @@ EXPORTS = [
     "smoe_peer_export", "smoe_peer_open", "smoe_peer_close", "smoe_xchg_publish", "smoe_grad_finalize_peers",
     "smoe_xchg_reduce_tail", "smoe_xchg_status", "smoe_feed", "smoe_halo_pull", "smoe_quant_ranges_bytes", "smoe_quant_ranges", "smoe_quant_route", "smoe_fake_quant_theta", "smoe_ssim_workspace_bytes", "smoe_ssim", "smoe_sqerr", "smoe_quantize", "smoe_rescale",
     "smoe_colminmax", "smoe_point_tiles", "smoe_point_stride", "smoe_point_plan_bytes", "smoe_point_splits",
-    "smoe_point_forward", "smoe_point_cotangent", "smoe_point_backward", "smoe_point_xgrad",
+    "smoe_point_forward", "smoe_point_cotangent", "smoe_point_backward", "smoe_point_xgrad", "smoe_point_jacobian",
+    "smoe_jacobian",
 ]
 
 

@@ -7,7 +7,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libsmoe_b200.so")
-SOURCES = ["pack.cu", "forward.cu", "backward.cu", "exchange.cu", "metrics.cu", "ssim_loss.cu", "points.cu"]
+SOURCES = ["pack.cu", "forward.cu", "backward.cu", "exchange.cu", "metrics.cu", "ssim_loss.cu", "points.cu", "jacobian.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared"]
 

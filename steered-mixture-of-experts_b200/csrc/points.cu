@@ -20,17 +20,11 @@
 // exactly zero (or absorbed, sweep A part 2), and every sum runs in a fixed order.  No float atomics anywhere.
 // A box with a NaN coordinate culls nothing: its thresholds become -inf (forward) and its min qthr NaN (backward,
 // coordinate gradient), and every culling comparison is written as !(bound < threshold).
-#include "smoe_common.cuh"
-#include "fwd_records.cuh"
+#include "pt_state.cuh"
 
 namespace smoe {
 
-constexpr int PP_QTHR = 0, PP_GR = 1, PP_G = 2;                      // then C planes g_c, then d planes x'_l
-__host__ __device__ constexpr int pp_x(int C) { return PP_G + C; }
-__host__ __device__ constexpr int pt_stride(int d, int C) { return (2 + C + d) * SMOE_TPIX; }
-constexpr int kTB = 8;                                                 // tile_box floats per tile
 constexpr int kPtMaxSplits = 256;
-constexpr float kLn2 = 0.69314718055994530942f;
 
 struct PtArgs {
     smoe_cfg cfg;
@@ -48,21 +42,6 @@ struct PtArgs {
     int n, ntiles, nwords, K_cap, num_splits, max_list, max_chunks;
     float ltau;
 };
-
-// tile-centred logit of one point, Horner: T + D FFMA
-template <int D, int C>
-__device__ __forceinline__ float point_logit(const float* __restrict__ f, const float (&x)[D]) {
-    using R = Rec<D, C>;
-    float q = f[R::OC];
-#pragma unroll
-    for (int l = 0; l < D; ++l) {
-        float t = f[R::OL + l];
-#pragma unroll
-        for (int m = l; m < D; ++m) t = fmaf(f[R::OQ + ut(D, l, m)], x[m], t);
-        q = fmaf(t, x[l], q);
-    }
-    return q;
-}
 
 // Box of the CTA's 512 points (first kThreadsF * PPT slots of the tile); x is made tile-centred in place.  `red`
 // holds 32 floats.  Returns true when some coordinate is NaN: the centre is then that of the other points (fminf /
@@ -951,20 +930,7 @@ __global__ void __launch_bounds__(kThreadsF, 4) point_xgrad_kernel(const PtArgs 
     }
 }
 
-template <int D, int C>
-static size_t pt_sweep_smem_bytes(int max_chunks) {
-    return (size_t)(2 * kChunk * pstride(D, C) + kChunk * Rec<D, C>::RC) * 4 + 2 * 8 + 32 * 4 + 8 * 4 +
-           (size_t)max_chunks * 4 + 64;
-}
-
-static int pt_tiles(int n) { return (int)(((long long)n + SMOE_TPIX - 1) / SMOE_TPIX); }
 static int pt_nwords(int ntiles) { return (ntiles + 127) / 128 * 4; }
-static int pt_sms() {
-    int dev = 0, sms = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    return sms;
-}
 
 }  // namespace smoe
 

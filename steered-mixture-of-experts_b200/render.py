@@ -190,7 +190,7 @@ class SmoeRenderer:
     and returns the mixture r before clip, shape (n0, n1[, n2], C).  Any of the tensors may require grad; gradients
     are zero where a variable is not read and for kernels with pi <= 0, as in the reference's graph.  Every call
     allocates its own state, so several renders can live in one autograd graph.  A render's backward runs once
-    (no retain_graph second pass)."""
+    (no retain_graph second pass).  `r.jacobian(params)` returns the render with its spatial Jacobian d r_c / d x_l."""
 
     def __init__(self, grid, channels=3, use_determinant=False, train_inverse_cov=False, precision=8, device=None,
                  _dense_exec=0):
@@ -209,14 +209,37 @@ class SmoeRenderer:
         self._axes = [torch.from_numpy(x).to(self.device) for x in axes]
 
     def __call__(self, params):
-        ts = check_params(params, self.d, self.C)
-        for k, t in zip(PARAM_KEYS, ts):
-            if t.device != self.device:
-                raise ValueError(f"params[{k!r}] is on {t.device}, the renderer on {self.device}")
+        ts = self._check(params)
         if torch.is_grad_enabled() and any(t.requires_grad for t in ts):
             return _Render.apply(self, *ts)
         with torch.cuda.device(self.device):
             return self._forward(ts, keep_state=False)[0]
+
+    def jacobian(self, params):
+        """(r, J): the mixture r before clip on the grid, (n0, n1[, n2], C), and its spatial Jacobian
+        J[..., c, l] = d r_c / d x_l, (n0, n1[, n2], C, d), per unit of model coordinate (not per pixel).
+
+        One forward and one CUDA sweep over the forward's per-pixel state (smoe_jacobian).  As with dL/dx of
+        `SmoePointRenderer`, the 0/1 gate decision w > tau contributes no term.  Both tensors are returned outside
+        autograd (requires_grad=False) whatever the params require: J is not differentiable.  Arguments are validated
+        as by a call; nothing synchronises with the host."""
+        ts = self._check(params)
+        with torch.no_grad(), torch.cuda.device(self.device):
+            out, state = self._forward(ts, keep_state=True)
+            theta, packed, indices, counts, pix, tile_qmin, chunk_bounds = state
+            jac = torch.empty(self.shape + (self.C, self.d), dtype=torch.float32, device=self.device)
+            check(lib().smoe_jacobian(C.byref(self._cfg), C.byref(self._batch), ptr(packed), ptr(counts),
+                                      ptr(chunk_bounds), theta.shape[0], ptr(pix), ptr(tile_qmin), *self._axis_ptrs(),
+                                      ptr(out), ptr(jac), stream_ptr()), "smoe_jacobian")
+        return out, jac
+
+    def _check(self, params):
+        """ValueError for params that __call__ and jacobian cannot take; returns the six parameter tensors."""
+        ts = check_params(params, self.d, self.C)
+        for k, t in zip(PARAM_KEYS, ts):
+            if t.device != self.device:
+                raise ValueError(f"params[{k!r}] is on {t.device}, the renderer on {self.device}")
+        return ts
 
     def _axis_ptrs(self):
         return (ptr(self._axes[0]), ptr(self._axes[1]), ptr(self._axes[2]) if self.d == 3 else ptr(None))
@@ -234,12 +257,12 @@ class SmoeRenderer:
         check(L.smoe_forward(C.byref(self._cfg), C.byref(self._batch), ptr(packed), ptr(indices), ptr(counts),
                              ptr(chunk_bounds), K, ptr(None), *self._axis_ptrs(), ptr(out), ptr(None), ptr(None),
                              ptr(pix), ptr(tile_qmin), ptr(None), st), "smoe_forward")
-        return out, (theta, packed, indices, counts, pix, tile_qmin)
+        return out, (theta, packed, indices, counts, pix, tile_qmin, chunk_bounds)
 
     def _backward(self, out, state, grad_out):
         """smoe_cotangent + smoe_backward + smoe_grad_finalize; returns the (K, P) gradient rows of theta."""
         L, st, dev = lib(), stream_ptr(), self.device
-        theta, packed, indices, counts, pix, tile_qmin = state
+        theta, packed, indices, counts, pix, tile_qmin, _ = state
         K, P = theta.shape
         check(L.smoe_cotangent(C.byref(self._cfg), C.byref(self._batch), ptr(out), ptr(grad_out), ptr(pix), st),
               "smoe_cotangent")
@@ -318,7 +341,8 @@ class SmoePointRenderer:
     never the result.  Coordinates must be finite: a NaN or infinite coordinate is the caller's responsibility (that
     point's values are undefined, and its tile of 512 points is evaluated without culling).  Nothing synchronises with the host.  Under
     no_grad no backward state is allocated; in the backward, the parameter sweep runs only when a parameter needs a
-    gradient and the coordinate sweep only when the points do.  A call's backward runs once."""
+    gradient and the coordinate sweep only when the points do.  A call's backward runs once.  `jacobian(params,
+    points)` returns r with its spatial Jacobian d r_c / d x_l."""
 
     def __init__(self, d=2, channels=3, use_determinant=False, train_inverse_cov=False, precision=8, device=None,
                  _dense_exec=0):
@@ -334,15 +358,40 @@ class SmoePointRenderer:
         self._key_scale = key_scale((1,) * self.d)         # model coordinates: one scale on every axis
 
     def __call__(self, params, points):
+        ts = self._check(params, points)
+        if torch.is_grad_enabled() and (points.requires_grad or any(t.requires_grad for t in ts)):
+            return _PointRender.apply(self, points, *ts)
+        with torch.cuda.device(self.device):
+            return self._forward(points, ts, keep_state=False)[0]
+
+    def jacobian(self, params, points):
+        """(r, J): the mixture r before clip at every point, (..., C), and its spatial Jacobian
+        J[..., c, l] = d r_c / d x_l, (..., C, d), both in the caller's order and per unit of model coordinate.
+
+        One forward and one CUDA sweep over the forward's state (smoe_point_jacobian) -- not C reverse passes.  As
+        with dL/dx, the 0/1 gate decision w > tau contributes no term.  Both tensors are returned outside autograd
+        (requires_grad=False) whatever the inputs require: J is not differentiable.  Arguments are validated as by a
+        call; nothing synchronises with the host."""
+        ts = self._check(params, points)
+        with torch.no_grad(), torch.cuda.device(self.device):
+            out, state = self._forward(points, ts, keep_state=True)
+            L, st = lib(), stream_ptr()
+            theta, packed, indices, counts, chunk_bounds, order, r, pstate, tile_box = state
+            n = r.shape[0]
+            jac = torch.empty((n, self.C, self.d), dtype=torch.float32, device=self.device)
+            check(L.smoe_point_jacobian(C.byref(self._cfg), ptr(packed), ptr(counts), ptr(chunk_bounds), theta.shape[0],
+                                        n, ptr(pstate), ptr(tile_box), ptr(r), ptr(jac), st), "smoe_point_jacobian")
+            J = torch.empty_like(jac).index_copy_(0, order, jac)
+        return out, J.reshape(points.shape[:-1] + (self.C, self.d))
+
+    def _check(self, params, points):
+        """ValueError for anything __call__ and jacobian cannot take; returns the six parameter tensors."""
         ts = check_params(params, self.d, self.C)
         for k, t in zip(PARAM_KEYS, ts):
             if t.device != self.device:
                 raise ValueError(f"params[{k!r}] is on {t.device}, the renderer on {self.device}")
         check_points(points, self.d, self.device)
-        if torch.is_grad_enabled() and (points.requires_grad or any(t.requires_grad for t in ts)):
-            return _PointRender.apply(self, points, *ts)
-        with torch.cuda.device(self.device):
-            return self._forward(points, ts, keep_state=False)[0]
+        return ts
 
     def _order(self, pts):
         """Stable Hilbert order of the points over their bounding box (one scale for every axis), on the device."""
