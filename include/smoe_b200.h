@@ -296,6 +296,30 @@ int smoe_jacobian(const smoe_cfg* cfg, const smoe_batch* batch, const float* pac
                   const float* chunk_bounds, int K_cap, const float* pix, const float* tile_qmin, const float* ax0,
                   const float* ax1, const float* ax2 /*NULL when d == 2*/, const float* rbuf, float* jac, void* stream);
 
+/* ---- Jacobian-vector products: forward-mode derivatives in the parameters and the points (csrc/jvp.cu) ------------
+ * dr = (d r / d theta) dtheta + (d r / d x) dpoints, the derivative of r before clip, in one pixel-stationary sweep
+ * after the forward, with the Jacobian's culling (the exact-zero cut), fixed packed-kernel order and no float atomics;
+ * cfg->dense_exec 0, 1 and 2 give the same bits.  As for dL/dx, the 0/1 gate decision w > tau contributes no term;
+ * kernels smoe_pack dropped (pi <= 0) have no tangent.  cfg->eps_bits must be 0.
+ *   smoe_pack_tangent  dtheta ([K_all][P], theta's row layout) -> tangent[K_cap][smoe_tangent_stride] in packed order,
+ *                      one record per packed row (read through `indices`; K from counts[0] on the device), for the
+ *                      theta, indices and counts of a smoe_pack call without fake quantisation or diff centres
+ *   smoe_jvp           dr in rbuf's layout on the grid of a smoe_forward call with pix / tile_qmin on `batch` (halo
+ *                      0), from its rbuf; call it before smoe_loss or smoe_cotangent (it reads the flag in gr)
+ *   smoe_point_jvp     dr[n][C] in tile order from the state, tile_box and r of a smoe_point_forward call with state;
+ *                      tangent (parameters) and dpoints ([n][d] tile order) may each be NULL, not both; call it before
+ *                      smoe_point_cotangent */
+int smoe_tangent_stride(int d, int C);      /* floats per record of `tangent` */
+int smoe_pack_tangent(const smoe_cfg* cfg, const float* theta, const float* dtheta, const int32_t* indices,
+                      const int32_t* counts, int K_cap, float* tangent, void* stream);
+int smoe_jvp(const smoe_cfg* cfg, const smoe_batch* batch, const float* packed, const float* tangent,
+             const int32_t* counts, const float* chunk_bounds, int K_cap, const float* pix, const float* tile_qmin,
+             const float* ax0, const float* ax1, const float* ax2 /*NULL when d == 2*/, const float* rbuf, float* dr,
+             void* stream);
+int smoe_point_jvp(const smoe_cfg* cfg, const float* packed, const float* tangent /*or NULL*/, const int32_t* counts,
+                   const float* chunk_bounds, int K_cap, int n_points, const float* state, const float* tile_box,
+                   const float* r, const float* dpoints /*[n][d] tile order, or NULL*/, float* dr, void* stream);
+
 /* Fixed-order reduction of the pixel splits: raw[k][j] = sum_s raw_part[s][k][j].  (The buffer a
  * multi-GPU run all-reduces with NCCL.) */
 int smoe_reduce_splits(const smoe_cfg* cfg, const int32_t* counts, int K_cap, int num_splits,

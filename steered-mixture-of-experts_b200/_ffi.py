@@ -27,7 +27,7 @@ EXPORTS = [
     "smoe_xchg_reduce_tail", "smoe_xchg_status", "smoe_feed", "smoe_halo_pull", "smoe_quant_ranges_bytes", "smoe_quant_ranges", "smoe_quant_route", "smoe_fake_quant_theta", "smoe_ssim_workspace_bytes", "smoe_ssim", "smoe_sqerr", "smoe_quantize", "smoe_rescale",
     "smoe_colminmax", "smoe_point_tiles", "smoe_point_stride", "smoe_point_plan_bytes", "smoe_point_splits",
     "smoe_point_forward", "smoe_point_cotangent", "smoe_point_backward", "smoe_point_xgrad", "smoe_point_jacobian",
-    "smoe_jacobian",
+    "smoe_jacobian", "smoe_tangent_stride", "smoe_pack_tangent", "smoe_jvp", "smoe_point_jvp",
 ]
 
 

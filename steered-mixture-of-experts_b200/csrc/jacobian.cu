@@ -19,146 +19,13 @@
 // forward computes them.  A thread's 4 pixels differ only in x'_0, so the logit is the forward's parabola, the
 // gradient along x'_0 is b + 2 qq00 x'_0 and along every other axis it is affine in x'_0: the parts that do not
 // depend on x'_0 are computed once per (thread, kernel).
-#include "pt_state.cuh"
+#include "jac_sweep.cuh"
 
 namespace smoe {
 
 // resident CTAs per SM: 4 (128 registers a thread) except at (3, 3), whose 36 accumulators, 12 coordinates, 12
 // f * r_c and 28-float record need 3 (168 registers)
 __host__ __device__ constexpr int jac_ctas(int d, int C) { return (d == 3 && C == 3) ? 3 : 4; }
-
-struct JacArgs {
-    smoe_cfg cfg;
-    smoe_batch b;              // smoe_jacobian only
-    const float* packed;
-    const int32_t* counts;
-    const float* chunk_bounds;
-    const float* state;        // smoe_point_jacobian: [ntiles][pt_stride], as smoe_point_forward left it;
-                               // smoe_jacobian: pix [ntiles][pix_stride], as smoe_forward left it
-    const float* tile_box;     // smoe_point_jacobian: [ntiles][kTB]; smoe_jacobian: tile_qmin [ntiles]
-    const float* ax[3];        // smoe_jacobian only
-    const float* r;            // [n][C]: tile order (points) or the grid's rbuf
-    float* jac;                // [n][C][d], the layout of r
-    int n, ntiles, nt1, nt2;
-    float ltau;
-};
-
-// Shared memory of a Jacobian sweep: two raw chunks, the compute records, barriers, `red`, `scratch`, chunk list.
-struct JacSmem {
-    float *raw0, *raw1, *crec;
-    uint64_t* bar;
-    int *scratch, *clist;
-    uint32_t phase0, phase1;
-    int par;
-};
-
-template <int D, int C>
-__device__ __forceinline__ JacSmem jac_smem_init() {
-    extern __shared__ __align__(128) unsigned char smem_raw[];
-    JacSmem s;
-    s.raw0 = reinterpret_cast<float*>(smem_raw);
-    s.raw1 = s.raw0 + kChunk * pstride(D, C);
-    s.crec = s.raw1 + kChunk * pstride(D, C);
-    s.bar = reinterpret_cast<uint64_t*>(s.crec + kChunk * Rec<D, C>::RC);
-    s.scratch = reinterpret_cast<int*>(reinterpret_cast<float*>(s.bar + 2) + 32);
-    s.clist = s.scratch + 8;
-    if (threadIdx.x == 0) {
-        mbar_init(&s.bar[0], 1);
-        mbar_init(&s.bar[1], 1);
-        fence_barrier_init();
-    }
-    __syncthreads();
-    s.phase0 = s.phase1 = 0;
-    s.par = 0;
-    return s;
-}
-
-// One tile's sweep, smoe_point_xgrad's staging and culling: the ordered list of chunks whose bound over the box
-// (ctr, half) reaches `thr`, TMA double buffering, per-kernel culling and ordered compaction; body(rec) is called for
-// every kernel that can matter, in packed order, with its tile-centred record.  Ends with a CTA barrier.
-template <int D, int C, class Body>
-__device__ __forceinline__ void jac_sweep(const JacArgs& a, JacSmem& s, int K, bool cull, const float (&ctr)[3],
-                                          const float (&half)[3], float thr, Body&& body) {
-    using R = Rec<D, C>;
-    constexpr int PK = pstride(D, C);
-    const int tid = threadIdx.x;
-    const int nchunks = (K + kChunk - 1) / kChunk;
-    auto issue = [&](int ci, int buf) {
-        int nk = min(kChunk, K - ci * kChunk);
-        uint32_t bytes = (uint32_t)nk * PK * 4u;
-        fence_proxy_async();
-        mbar_expect_tx(&s.bar[buf], bytes);
-        tma_load_1d(buf ? s.raw1 : s.raw0, a.packed + (size_t)ci * kChunk * PK, bytes, &s.bar[buf]);
-    };
-    int nlist = 0;
-    for (int base = 0; base < nchunks; base += kThreadsF) {
-        const int ci = base + tid;
-        bool need = ci < nchunks;
-        if (need && cull) {
-            const float* cb = a.chunk_bounds + (size_t)ci * kCB;
-            float d2 = 0.f, kd = 0.f;
-#pragma unroll
-            for (int l = 0; l < D; ++l) {
-                const float mn = cb[l] - ctr[l], mx = cb[3 + l] - ctr[l];
-                const float gap = fmaxf(fmaxf(mn - half[l], -half[l] - mx), 0.f);
-                d2 = fmaf(gap, gap, d2);
-                kd = fmaxf(kd, cb[8 + l] * gap * gap);
-            }
-            const float lam = cb[6];
-            need = !(lam >= 0.f) || !(cb[7] - fmaxf(lam * d2, kd) < thr);
-        }
-        int tot;
-        const int pos = cta_compact(need, s.scratch, s.par, &tot);
-        if (need) s.clist[nlist + pos] = ci;
-        nlist += tot;
-    }
-    __syncthreads();
-
-    if (tid == 0 && nlist > 0) {
-        issue(s.clist[0], 0);
-        if (nlist > 1) issue(s.clist[1], 1);
-    }
-    for (int li = 0; li < nlist; ++li) {
-        const int buf = li & 1;
-        const int ci = s.clist[li];
-        const int nk = min(kChunk, K - ci * kChunk);
-        if (buf) { mbar_wait(&s.bar[1], s.phase1); s.phase1 ^= 1; } else { mbar_wait(&s.bar[0], s.phase0); s.phase0 ^= 1; }
-        const float* raw = (buf ? s.raw1 : s.raw0) + tid * PK;
-        bool need = tid < nk;
-        float mu[D];
-#pragma unroll
-        for (int l = 0; l < D; ++l) mu[l] = need ? raw[off_mu(D, C) + l] - ctr[l] : 0.f;
-        if (need && cull) {
-            float d2 = 0.f, kd = 0.f;
-#pragma unroll
-            for (int l = 0; l < D; ++l) {
-                const float gap = fmaxf(fabsf(mu[l]) - half[l], 0.f);
-                d2 = fmaf(gap, gap, d2);
-                kd = fmaxf(kd, raw[nparam(D, C) + 1 + l] * gap * gap);
-            }
-            const float lam = raw[nparam(D, C)];
-            need = !(lam >= 0.f) || !(raw[off_pi(D, C)] - fmaxf(lam * d2, kd) < thr);
-        }
-        int nneed;
-        const int pos = cta_compact(need, s.scratch, s.par, &nneed);
-        if (need) transform_record<D, C>(raw, mu, ctr, 0, s.crec + pos * R::RC);
-        __syncthreads();
-        if (tid == 0 && li + 2 < nlist) issue(s.clist[li + 2], buf);
-        for (int kk = 0; kk < nneed; ++kk) body(s.crec + kk * R::RC);
-    }
-    __syncthreads();          // the next tile rebuilds `clist` and re-uses `crec`
-}
-
-// record -> registers: the geometry part (NG4 float4), or the rest up to the original index
-template <int D, int C>
-__device__ __forceinline__ void load_rec(const float* rc, float (&f)[Rec<D, C>::RC], int from, int to) {
-    const float4* r4 = reinterpret_cast<const float4*>(rc);
-#pragma unroll
-    for (int j = from; j < to; ++j) {
-        float4 v = r4[j];
-        f[4 * j] = v.x; f[4 * j + 1] = v.y; f[4 * j + 2] = v.z; f[4 * j + 3] = v.w;
-    }
-}
 
 template <int D, int C>
 __global__ void __launch_bounds__(kThreadsF, jac_ctas(D, C)) point_jacobian_kernel(const JacArgs a) {

@@ -29,6 +29,7 @@ from collections.abc import Mapping
 
 import numpy as np
 import torch
+import torch.autograd.forward_ad as fwAD
 from torch.autograd.function import once_differentiable
 
 from . import _ffi
@@ -126,17 +127,24 @@ def make_cfg(d, C_, precision, use_determinant, train_inverse_cov, dense_exec):
                q_ub=(C.c_float * 5)(*[1.0] * 5), q_bits=(C.c_int32 * 5)(*[8] * 5), dense_exec=int(dense_exec))
 
 
+def theta_rows(ts, d):
+    """The six parameter tensors (PARAM_KEYS order) -> (K, P) theta rows: musX | the diagonal of A_diagonal and the
+    strictly-lower part of A_corr, row by row | pis | nu_e | gamma_e.  The entries the op never reads are dropped."""
+    pis, musX, A_diag, A_corr, gamma_e, nu_e = ts
+    K = pis.shape[0]
+    A_cols = torch.stack([A_diag[:, l, l] if l == m else A_corr[:, l, m] for l in range(d) for m in range(l + 1)], 1)
+    return torch.cat([musX, A_cols, pis[:, None], nu_e, gamma_e.reshape(K, -1)], 1).contiguous()
+
+
 def pack_model(cfg, ts, scale):
     """The six parameter tensors -> theta rows, Hilbert keys of the centres (smoe_spatial_keys, per-axis `scale`), a
     stable sort and smoe_pack on the current stream.  Returns (theta, packed, indices, counts, chunk_bounds)."""
     L, st, f32, i32 = lib(), stream_ptr(), torch.float32, torch.int32
     d, Cc = cfg.d, cfg.C
     P, PK = L.smoe_param_count(d, Cc), L.smoe_packed_stride(d, Cc)
-    pis, musX, A_diag, A_corr, gamma_e, nu_e = (t.detach() for t in ts)
-    dev = pis.device
-    K = pis.shape[0]
-    A_cols = torch.stack([A_diag[:, l, l] if l == m else A_corr[:, l, m] for l in range(d) for m in range(l + 1)], 1)
-    theta = torch.cat([musX, A_cols, pis[:, None], nu_e, gamma_e.reshape(K, d * Cc)], 1).contiguous()
+    theta = theta_rows([t.detach() for t in ts], d)
+    dev = theta.device
+    K = theta.shape[0]
     keys = torch.empty((K,), dtype=torch.int64, device=dev)
     check(L.smoe_spatial_keys(ptr(theta), K, d, P, ptr(None), scale, ptr(keys), st), "smoe_spatial_keys")
     perm = torch.sort(keys, stable=True).indices.to(i32)
@@ -152,6 +160,56 @@ def pack_model(cfg, ts, scale):
                       ptr(packed), ptr(indices), ptr(pos), ptr(counts), ptr(regsums), ptr(chunk_bounds), ptr(ws),
                       ptr(None), ptr(None), ptr(None), st), "smoe_pack")
     return theta, packed, indices, counts, chunk_bounds
+
+
+def tangent_rows(dts, K, d, Cc, device):
+    """Forward-mode tangents of the six parameter tensors (None: no tangent) -> their (K, P) theta rows; raises
+    ValueError for a shape or device that does not match the parameter's."""
+    expect = dict(pis=(K,), musX=(K, d), A_diagonal=(K, d, d), A_corr=(K, d, d), gamma_e=(K, d, Cc), nu_e=(K, Cc))
+    rows = []
+    for k, dt in zip(PARAM_KEYS, dts):
+        if dt is None:
+            dt = torch.zeros(expect[k], dtype=torch.float32, device=device)
+        elif tuple(dt.shape) != expect[k] or dt.device != device:
+            raise ValueError(f"the tangent of {k!r} must have shape {expect[k]} on {device}, got "
+                             f"{tuple(dt.shape)} on {dt.device}")
+        rows.append(plain(dt).to(torch.float32))
+    return theta_rows(rows, d)
+
+
+def plain(t):
+    """The device tensor under a `torch.func` transform's wrappers (a tangent or a saved output inside `jvp`),
+    detached: the CUDA calls take its data pointer.  Used under torch._C._DisableFuncTorch(), so that the tensors the
+    JVP computes from it stay plain too."""
+    while torch._C._functorch.is_functorch_wrapped_tensor(t):
+        t = torch._C._functorch.get_unwrapped(t)
+    return t.detach()
+
+
+def pack_tangent(cfg, theta, dts, indices, counts):
+    """smoe_pack_tangent on the current stream: the parameter tangents -> one tangent record per packed row."""
+    L = lib()
+    K = theta.shape[0]
+    dtheta = tangent_rows(dts, K, cfg.d, cfg.C, theta.device)
+    tangent = torch.empty((K, L.smoe_tangent_stride(cfg.d, cfg.C)), dtype=torch.float32, device=theta.device)
+    check(L.smoe_pack_tangent(C.byref(cfg), ptr(theta), ptr(dtheta), ptr(indices), ptr(counts), K, ptr(tangent),
+                              stream_ptr()), "smoe_pack_tangent")
+    return tangent
+
+
+def traced(ts):
+    """Whether a call must go through autograd: grad mode is on and a tensor requires grad, or a tensor carries a
+    forward-mode tangent (a `forward_ad` dual tensor or a `torch.func` transform's tensor), which the no-grad fast
+    path would drop."""
+    if torch.is_grad_enabled() and any(t.requires_grad for t in ts):
+        return True
+    return any(torch._C._functorch.is_functorch_wrapped_tensor(t) or fwAD.unpack_dual(t).tangent is not None
+               for t in ts)
+
+
+class _Slot:
+    """Hands a call's device state from an autograd Function's forward to its setup_context."""
+    __slots__ = ("state",)
 
 
 def finalize_grads(cfg, raw_part, splits, plan, theta, indices, counts):
@@ -190,7 +248,13 @@ class SmoeRenderer:
     and returns the mixture r before clip, shape (n0, n1[, n2], C).  Any of the tensors may require grad; gradients
     are zero where a variable is not read and for kernels with pi <= 0, as in the reference's graph.  Every call
     allocates its own state, so several renders can live in one autograd graph.  A render's backward runs once
-    (no retain_graph second pass).  `r.jacobian(params)` returns the render with its spatial Jacobian d r_c / d x_l."""
+    (no retain_graph second pass).  `r.jacobian(params)` returns the render with its spatial Jacobian d r_c / d x_l.
+
+    Forward mode: under `torch.func.jvp` or with `torch.autograd.forward_ad` dual tensors a call also returns the
+    Jacobian-vector product dr = (d r / d params) . tangents, from one more CUDA sweep after the forward
+    (smoe_pack_tangent + smoe_jvp); r is the plain call's, and the call's backward, if any, is unchanged.  As in
+    reverse mode, tangents of kernels with pi <= 0 and of entries the op does not read have no effect, and the 0/1
+    gate decision w > tau contributes no term.  `torch.func.vmap` / `jacfwd` have no batching rule."""
 
     def __init__(self, grid, channels=3, use_determinant=False, train_inverse_cov=False, precision=8, device=None,
                  _dense_exec=0):
@@ -210,8 +274,8 @@ class SmoeRenderer:
 
     def __call__(self, params):
         ts = self._check(params)
-        if torch.is_grad_enabled() and any(t.requires_grad for t in ts):
-            return _Render.apply(self, *ts)
+        if traced(ts):
+            return _Render.apply(self, _Slot(), *ts)
         with torch.cuda.device(self.device):
             return self._forward(ts, keep_state=False)[0]
 
@@ -275,16 +339,38 @@ class SmoeRenderer:
               "smoe_backward")
         return finalize_grads(self._cfg, raw_part, splits, plan, theta, indices, counts)
 
+    def _jvp(self, out, state, dts):
+        """smoe_pack_tangent + smoe_jvp after the forward that left `state`: dr for the parameter tangents dts."""
+        theta, packed, indices, counts, pix, tile_qmin, chunk_bounds = state
+        tangent = pack_tangent(self._cfg, theta, dts, indices, counts)
+        dr = torch.empty_like(out)
+        check(lib().smoe_jvp(C.byref(self._cfg), C.byref(self._batch), ptr(packed), ptr(tangent), ptr(counts),
+                             ptr(chunk_bounds), theta.shape[0], ptr(pix), ptr(tile_qmin), *self._axis_ptrs(), ptr(out),
+                             ptr(dr), stream_ptr()), "smoe_jvp")
+        return dr
+
 
 class _Render(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, renderer, *ts):
+    def forward(renderer, slot, *ts):
         with torch.cuda.device(renderer.device):
-            out, state = renderer._forward(ts, keep_state=True)
-        ctx.renderer = renderer
-        ctx.state = state
-        ctx.save_for_backward(out)
+            out, slot.state = renderer._forward(ts, keep_state=True)
         return out
+
+    @staticmethod
+    def setup_context(ctx, inputs, output):
+        ctx.renderer = inputs[0]
+        ctx.state = inputs[1].state
+        ctx.set_materialize_grads(False)
+        ctx.save_for_backward(output)
+        ctx.save_for_forward(output)
+
+    @staticmethod
+    def jvp(ctx, _renderer, _slot, *dts):
+        (out,) = ctx.saved_tensors
+        r = ctx.renderer
+        with torch._C._DisableFuncTorch(), torch.cuda.device(r.device):
+            return r._jvp(plain(out), ctx.state, dts)
 
     @staticmethod
     @once_differentiable
@@ -298,7 +384,7 @@ class _Render(torch.autograd.Function):
             grads = r._backward(out, ctx.state, grad_out.to(torch.float32).contiguous())
             ctx.state = None
             parts = split_grads(grads, r.d, r.C)
-        return (None,) + tuple(g if need else None for g, need in zip(parts, ctx.needs_input_grad[1:]))
+        return (None, None) + tuple(g if need else None for g, need in zip(parts, ctx.needs_input_grad[2:]))
 
 
 MAX_POINTS = 2147483136        # SMOE_POINT_MAX: point indices of the tiles stay below 2^31
@@ -342,7 +428,11 @@ class SmoePointRenderer:
     point's values are undefined, and its tile of 512 points is evaluated without culling).  Nothing synchronises with the host.  Under
     no_grad no backward state is allocated; in the backward, the parameter sweep runs only when a parameter needs a
     gradient and the coordinate sweep only when the points do.  A call's backward runs once.  `jacobian(params,
-    points)` returns r with its spatial Jacobian d r_c / d x_l."""
+    points)` returns r with its spatial Jacobian d r_c / d x_l.
+
+    Forward mode: under `torch.func.jvp` or with `torch.autograd.forward_ad` dual tensors, with tangents on the params
+    and/or the points, a call also returns dr = (d r / d params) . v + (d r / d x) . xdot from one more CUDA sweep
+    after the forward (smoe_pack_tangent when the params carry tangents, then smoe_point_jvp), as `SmoeRenderer`."""
 
     def __init__(self, d=2, channels=3, use_determinant=False, train_inverse_cov=False, precision=8, device=None,
                  _dense_exec=0):
@@ -359,8 +449,8 @@ class SmoePointRenderer:
 
     def __call__(self, params, points):
         ts = self._check(params, points)
-        if torch.is_grad_enabled() and (points.requires_grad or any(t.requires_grad for t in ts)):
-            return _PointRender.apply(self, points, *ts)
+        if traced((points,) + ts):
+            return _PointRender.apply(self, _Slot(), points, *ts)
         with torch.cuda.device(self.device):
             return self._forward(points, ts, keep_state=False)[0]
 
@@ -447,16 +537,46 @@ class SmoePointRenderer:
             gx = torch.empty_like(gs).index_copy_(0, order, gs)
         return grads, gx
 
+    def _jvp(self, state, dpoints, dts):
+        """smoe_pack_tangent (parameter tangents) + smoe_point_jvp after the forward that left `state`: dr (N, C) in
+        the caller's order for the parameter tangents dts and the point tangents dpoints (None: none)."""
+        L, dev, f32 = lib(), self.device, torch.float32
+        theta, packed, indices, counts, chunk_bounds, order, r, pstate, tile_box = state
+        n = r.shape[0]
+        if dpoints is None and all(dt is None for dt in dts):
+            return torch.zeros_like(r)
+        tangent = pack_tangent(self._cfg, theta, dts, indices, counts) if any(dt is not None for dt in dts) else None
+        dxs = None
+        if dpoints is not None:
+            if dpoints.numel() != n * self.d or dpoints.device != dev:
+                raise ValueError(f"the tangent of the points must have {n} x {self.d} values on {dev}")
+            dxs = plain(dpoints).to(f32).reshape(-1, self.d).index_select(0, order).contiguous()
+        drs = torch.empty((n, self.C), dtype=f32, device=dev)
+        check(L.smoe_point_jvp(C.byref(self._cfg), ptr(packed), ptr(tangent), ptr(counts), ptr(chunk_bounds),
+                               theta.shape[0], n, ptr(pstate), ptr(tile_box), ptr(r), ptr(dxs), ptr(drs),
+                               stream_ptr()), "smoe_point_jvp")
+        return torch.empty_like(drs).index_copy_(0, order, drs)
+
 
 class _PointRender(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, renderer, points, *ts):
+    def forward(renderer, slot, points, *ts):
         with torch.cuda.device(renderer.device):
-            out, state = renderer._forward(points, ts, keep_state=True)
-        ctx.renderer = renderer
-        ctx.state = state
-        ctx.points_shape = points.shape
+            out, slot.state = renderer._forward(points, ts, keep_state=True)
         return out
+
+    @staticmethod
+    def setup_context(ctx, inputs, output):
+        ctx.renderer = inputs[0]
+        ctx.state = inputs[1].state
+        ctx.points_shape = inputs[2].shape
+        ctx.set_materialize_grads(False)
+
+    @staticmethod
+    def jvp(ctx, _renderer, _slot, dpoints, *dts):
+        r = ctx.renderer
+        with torch._C._DisableFuncTorch(), torch.cuda.device(r.device):
+            return r._jvp(ctx.state, dpoints, dts).reshape(ctx.points_shape[:-1] + (r.C,))
 
     @staticmethod
     @once_differentiable
@@ -465,10 +585,10 @@ class _PointRender(torch.autograd.Function):
             raise RuntimeError("SmoePointRenderer: a call's backward runs once (smoe_point_cotangent consumes the "
                                "forward's point state); evaluate again for another backward pass")
         r = ctx.renderer
-        need_points, need_params = ctx.needs_input_grad[1], any(ctx.needs_input_grad[2:])
+        need_points, need_params = ctx.needs_input_grad[2], any(ctx.needs_input_grad[3:])
         with torch.cuda.device(r.device):
             grads, gx = r._backward(ctx.state, grad_out.to(torch.float32).contiguous(), need_params, need_points)
             ctx.state = None
             parts = split_grads(grads, r.d, r.C) if grads is not None else (None,) * len(PARAM_KEYS)
-        return ((None, gx.reshape(ctx.points_shape) if gx is not None else None)
-                + tuple(g if need else None for g, need in zip(parts, ctx.needs_input_grad[2:])))
+        return ((None, None, gx.reshape(ctx.points_shape) if gx is not None else None)
+                + tuple(g if need else None for g, need in zip(parts, ctx.needs_input_grad[3:])))
