@@ -320,6 +320,48 @@ int smoe_point_jvp(const smoe_cfg* cfg, const float* packed, const float* tangen
                    const float* chunk_bounds, int K_cap, int n_points, const float* state, const float* tile_box,
                    const float* r, const float* dpoints /*[n][d] tile order, or NULL*/, float* dr, void* stream);
 
+/* ---- Gauss-Newton diagonal: D = diag(J^T diag(h) J) in every parameter (csrc/gn_diag.cu) -------------------------
+ * J = d r / d theta of r before clip, h >= 0 a per-sample, per-channel weight (NULL: h = 1, so D = diag(J^T J); for a
+ * loss sum l(r), h = l'' gives the generalised Gauss-Newton diagonal).  Per kernel, P non-negative sums over the
+ * samples: ln2^2 w^2 (dq/dtheta_i)^2 sum_c h_c (m E_c - f r_c)^2 for the gate parameters (mu, the A entries the op
+ * reads, pi; dq/dtheta_i as smoe_pack_tangent's one-hot tangent logit), h_c m w^2 for nu and h_c m w^2 x_l^2 for gamma.
+ * As for the JVP, the 0/1 gate decision w > tau contributes no term and kernels smoe_pack dropped (pi <= 0) have no
+ * row.  Kernel-stationary sweep after the forward, with backward_kernel's CTAs, splits and planning pre-pass, no float
+ * atomics; cfg->dense_exec 0, 1 and 2 give the same bits.  cfg->eps_bits must be 0; no fake quantisation, diff
+ * centres or radial A.  Four stages, in stream order:
+ *   smoe_gn_state          after smoe_forward with pix / tile_qmin on `batch` (halo 0) and BEFORE smoe_loss or
+ *                          smoe_cotangent, which overwrite the flag S > 1e-11 in the gr plane: writes gstate, per tile
+ *                          of smoe_gn_state_stride floats: planes z | qthr | h_c | f r_c of SMOE_TPIX floats, then the
+ *                          row coordinates of pix.  weight[sample * stride_sample + c * stride_channel] with sample the
+ *                          pixel index of rbuf's layout (strides 0 broadcast), or NULL
+ *   smoe_point_gn_state    the same after smoe_point_forward with state, before smoe_point_cotangent: planes
+ *                          qthr | h_c | f r_c | x'_l per tile of smoe_point_gn_state_stride floats.  r in tile order;
+ *                          the weight is indexed by the caller's row order[i] ([n] int64) of tile slot i
+ *   smoe_gn_diag /         planning pre-pass (bwd_plan_kernel / point_plan_kernel) + sweep into raw_part
+ *   smoe_point_gn_diag     [num_splits][K_cap][P] in theta's column layout (mu | A lower-tri | pi | nu | gamma), packed
+ *                          order, and `plan` (smoe_backward_plan_bytes / smoe_point_plan_bytes; num_splits as for
+ *                          smoe_backward / smoe_point_splits).  theta and indices are those of the smoe_pack call.
+ *   then smoe_reduce_splits(raw_part, plan) -> raw[K_cap][P], and
+ *   smoe_gn_diag_scatter   diag[indices[k]] = raw[k] for the counts[0] packed rows (K on the device); the caller zeroes
+ *                          diag[K_all][P] first, so dropped kernels keep 0 rows. */
+int smoe_gn_state_stride(int d, int C, const smoe_batch* batch);     /* floats of gstate per grid tile */
+int smoe_point_gn_state_stride(int d, int C);                        /* floats of gstate per point tile */
+int smoe_gn_state(const smoe_cfg* cfg, const smoe_batch* batch, const float* pix, const float* rbuf,
+                  const float* weight /*or NULL*/, long long weight_stride_sample, long long weight_stride_channel,
+                  float* gstate, void* stream);
+int smoe_point_gn_state(const smoe_cfg* cfg, int n_points, const float* state, const float* r,
+                        const float* weight /*or NULL*/, const int64_t* order /*with a weight*/,
+                        long long weight_stride_sample, long long weight_stride_channel, float* gstate, void* stream);
+int smoe_gn_diag(const smoe_cfg* cfg, const smoe_batch* batch, const float* packed, const float* theta,
+                 const int32_t* indices, const int32_t* counts, int K_cap, const float* gstate, const float* tile_qmin,
+                 const float* ax0, const float* ax1, const float* ax2 /*NULL when d == 2*/, int num_splits,
+                 float* raw_part, int32_t* plan, void* stream);
+int smoe_point_gn_diag(const smoe_cfg* cfg, const float* packed, const float* theta, const int32_t* indices,
+                       const int32_t* counts, int K_cap, int n_points, const float* gstate, const float* tile_box,
+                       int num_splits, float* raw_part, int32_t* plan, void* stream);
+int smoe_gn_diag_scatter(const smoe_cfg* cfg, const float* raw, const int32_t* indices, const int32_t* counts,
+                         int K_cap, float* diag, void* stream);
+
 /* Fixed-order reduction of the pixel splits: raw[k][j] = sum_s raw_part[s][k][j].  (The buffer a
  * multi-GPU run all-reduces with NCCL.) */
 int smoe_reduce_splits(const smoe_cfg* cfg, const int32_t* counts, int K_cap, int num_splits,

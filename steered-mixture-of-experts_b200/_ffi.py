@@ -28,6 +28,8 @@ EXPORTS = [
     "smoe_colminmax", "smoe_point_tiles", "smoe_point_stride", "smoe_point_plan_bytes", "smoe_point_splits",
     "smoe_point_forward", "smoe_point_cotangent", "smoe_point_backward", "smoe_point_xgrad", "smoe_point_jacobian",
     "smoe_jacobian", "smoe_tangent_stride", "smoe_pack_tangent", "smoe_jvp", "smoe_point_jvp",
+    "smoe_gn_state_stride", "smoe_point_gn_state_stride", "smoe_gn_state", "smoe_point_gn_state", "smoe_gn_diag",
+    "smoe_point_gn_diag", "smoe_gn_diag_scatter",
 ]
 
 

@@ -235,6 +235,49 @@ def split_grads(grads, d, Cc):
             grads[:, o["ga"]:].reshape(K, d, Cc).contiguous(), grads[:, o["nu"]:o["nu"] + Cc].contiguous())
 
 
+def check_weight(weight, shape, device):
+    """The Gauss-Newton weight h, broadcastable to r's `shape` (..., C) -> (a (samples, C) view or copy, its sample
+    stride, its channel stride), or (None, 0, 0) for h = 1; raises ValueError for a type, dtype, device or shape the
+    call cannot take.  The values are not checked (that would synchronise)."""
+    if weight is None:
+        return None, 0, 0
+    if not isinstance(weight, torch.Tensor):
+        raise ValueError(f"weight must be a torch.Tensor or None, got {type(weight).__name__}")
+    if weight.dtype != torch.float32:
+        raise ValueError(f"weight must be float32, got {weight.dtype}")
+    if weight.device != device:
+        raise ValueError(f"weight is on {weight.device}, the renderer on {device}")
+    try:
+        ok = torch.broadcast_shapes(tuple(weight.shape), tuple(shape)) == tuple(shape)
+    except RuntimeError:
+        ok = False
+    if not ok:
+        raise ValueError(f"weight of shape {tuple(weight.shape)} does not broadcast to r's shape {tuple(shape)}")
+    w = weight.detach().expand(tuple(shape))
+    try:
+        w = w.view(-1, shape[-1])                  # per-sample, per-channel or full weights need no copy
+    except RuntimeError:
+        w = w.reshape(-1, shape[-1]).contiguous()
+    return w, w.stride(0), w.stride(1)
+
+
+def weight_args(w, ss, sc):
+    return (C.c_void_p(w.data_ptr()) if w is not None else ptr(None)), C.c_longlong(ss), C.c_longlong(sc)
+
+
+def gn_finalize(cfg, raw_part, splits, plan, indices, counts, K, P):
+    """smoe_reduce_splits + smoe_gn_diag_scatter: the split slabs of a Gauss-Newton diagonal sweep -> (K, P) rows in
+    theta's layout and original kernel order, zero for kernels with pi <= 0."""
+    L, st, dev = lib(), stream_ptr(), raw_part.device
+    raw = torch.empty((K, P), dtype=torch.float32, device=dev)
+    check(L.smoe_reduce_splits(C.byref(cfg), ptr(counts), K, splits, ptr(raw_part), ptr(plan), ptr(raw), st),
+          "smoe_reduce_splits")
+    diag = torch.zeros((K, P), dtype=torch.float32, device=dev)
+    check(L.smoe_gn_diag_scatter(C.byref(cfg), ptr(raw), ptr(indices), ptr(counts), K, ptr(diag), st),
+          "smoe_gn_diag_scatter")
+    return diag
+
+
 class SmoeRenderer:
     """Differentiable render of an SMoE on a uniform grid; see the module docstring.
 
@@ -254,7 +297,8 @@ class SmoeRenderer:
     Jacobian-vector product dr = (d r / d params) . tangents, from one more CUDA sweep after the forward
     (smoe_pack_tangent + smoe_jvp); r is the plain call's, and the call's backward, if any, is unchanged.  As in
     reverse mode, tangents of kernels with pi <= 0 and of entries the op does not read have no effect, and the 0/1
-    gate decision w > tau contributes no term.  `torch.func.vmap` / `jacfwd` have no batching rule."""
+    gate decision w > tau contributes no term.  `torch.func.vmap` / `jacfwd` have no batching rule.
+    `r.gauss_newton_diagonal(params, weight=None)` returns the render with diag(J^T diag(h) J) in every parameter."""
 
     def __init__(self, grid, channels=3, use_determinant=False, train_inverse_cov=False, precision=8, device=None,
                  _dense_exec=0):
@@ -296,6 +340,40 @@ class SmoeRenderer:
                                       ptr(chunk_bounds), theta.shape[0], ptr(pix), ptr(tile_qmin), *self._axis_ptrs(),
                                       ptr(out), ptr(jac), stream_ptr()), "smoe_jacobian")
         return out, jac
+
+    def gauss_newton_diagonal(self, params, weight=None):
+        """(r, D): the mixture r before clip on the grid, (n0, n1[, n2], C), bitwise the plain call's, and the
+        Gauss-Newton diagonal D = diag(J^T diag(h) J) of J = d r / d params, a dict in the params' layout and dtype.
+
+        `weight` is h, a float32 tensor on the renderer's device broadcastable to r's shape (per sample, per channel or
+        both), or None for h = 1, which gives diag(J^T J).  For a loss sum_n,c l(r_c(x_n)), h = l'' gives the
+        generalised Gauss-Newton diagonal; for 1/2 |r - y|^2 it is 1.  D is exact for whatever h is given: a Jacobi
+        preconditioner for CG, Marquardt's scaling for Levenberg-Marquardt, or the sensitivity of the loss to each
+        parameter.  As for the JVP, the 0/1 gate decision w > tau contributes no term; entries the op does not read
+        and the rows of kernels with pi <= 0 are 0.  One forward, an elementwise state stage and one kernel-stationary
+        CUDA sweep (smoe_gn_state, smoe_gn_diag, smoe_reduce_splits, smoe_gn_diag_scatter).  Both results are returned
+        outside autograd.  Arguments are validated as by a call, and `weight`'s shape, dtype and device too; its
+        values are not.  Nothing synchronises with the host."""
+        ts = self._check(params)
+        w, ss, sc = check_weight(weight, self.shape + (self.C,), self.device)
+        with torch.no_grad(), torch.cuda.device(self.device):
+            out, state = self._forward(ts, keep_state=True)
+            L, st, dev = lib(), stream_ptr(), self.device
+            theta, packed, indices, counts, pix, tile_qmin, _ = state
+            K, P = theta.shape
+            gstate = torch.empty((self._ntiles * L.smoe_gn_state_stride(self.d, self.C, C.byref(self._batch)),),
+                                 dtype=torch.float32, device=dev)
+            check(L.smoe_gn_state(C.byref(self._cfg), C.byref(self._batch), ptr(pix), ptr(out), *weight_args(w, ss, sc),
+                                  ptr(gstate), st), "smoe_gn_state")
+            splits = backward_splits(K, [self._batch])
+            raw_part = torch.empty((splits * K * P,), dtype=torch.float32, device=dev)
+            plan = torch.empty(((L.smoe_backward_plan_bytes(K, C.byref(self._batch)) + 3) // 4,), dtype=torch.int32,
+                               device=dev)
+            check(L.smoe_gn_diag(C.byref(self._cfg), C.byref(self._batch), ptr(packed), ptr(theta), ptr(indices),
+                                 ptr(counts), K, ptr(gstate), ptr(tile_qmin), *self._axis_ptrs(), splits, ptr(raw_part),
+                                 ptr(plan), st), "smoe_gn_diag")
+            diag = gn_finalize(self._cfg, raw_part, splits, plan, indices, counts, K, P)
+        return out, dict(zip(PARAM_KEYS, split_grads(diag, self.d, self.C)))
 
     def _check(self, params):
         """ValueError for params that __call__ and jacobian cannot take; returns the six parameter tensors."""
@@ -432,7 +510,8 @@ class SmoePointRenderer:
 
     Forward mode: under `torch.func.jvp` or with `torch.autograd.forward_ad` dual tensors, with tangents on the params
     and/or the points, a call also returns dr = (d r / d params) . v + (d r / d x) . xdot from one more CUDA sweep
-    after the forward (smoe_pack_tangent when the params carry tangents, then smoe_point_jvp), as `SmoeRenderer`."""
+    after the forward (smoe_pack_tangent when the params carry tangents, then smoe_point_jvp), as `SmoeRenderer`.
+    `gauss_newton_diagonal(params, points, weight=None)` returns r with diag(J^T diag(h) J) in every parameter."""
 
     def __init__(self, d=2, channels=3, use_determinant=False, train_inverse_cov=False, precision=8, device=None,
                  _dense_exec=0):
@@ -473,6 +552,35 @@ class SmoePointRenderer:
                                         n, ptr(pstate), ptr(tile_box), ptr(r), ptr(jac), st), "smoe_point_jacobian")
             J = torch.empty_like(jac).index_copy_(0, order, jac)
         return out, J.reshape(points.shape[:-1] + (self.C, self.d))
+
+    def gauss_newton_diagonal(self, params, points, weight=None):
+        """(r, D): the mixture r before clip at every point, (..., C) in the caller's order and bitwise the plain
+        call's, and the Gauss-Newton diagonal D = diag(J^T diag(h) J) of J = d r / d params, a dict in the params'
+        layout and dtype.  `weight` (h) is broadcastable to r's shape, or None for h = 1; see
+        `SmoeRenderer.gauss_newton_diagonal`.  One forward, an elementwise state stage and one kernel-stationary CUDA
+        sweep (smoe_point_gn_state, smoe_point_gn_diag, smoe_reduce_splits, smoe_gn_diag_scatter), outside autograd;
+        nothing synchronises with the host."""
+        ts = self._check(params, points)
+        w, ss, sc = check_weight(weight, tuple(points.shape[:-1]) + (self.C,), self.device)
+        with torch.no_grad(), torch.cuda.device(self.device):
+            out, state = self._forward(points, ts, keep_state=True)
+            L, st, dev = lib(), stream_ptr(), self.device
+            theta, packed, indices, counts, chunk_bounds, order, r, pstate, tile_box = state
+            K, P = theta.shape
+            n = r.shape[0]
+            gstate = torch.empty((L.smoe_point_tiles(n) * L.smoe_point_gn_state_stride(self.d, self.C),),
+                                 dtype=torch.float32, device=dev)
+            wp, wss, wsc = weight_args(w, ss, sc)
+            check(L.smoe_point_gn_state(C.byref(self._cfg), n, ptr(pstate), ptr(r), wp, ptr(order), wss, wsc,
+                                        ptr(gstate), st), "smoe_point_gn_state")
+            splits = L.smoe_point_splits(K, n)
+            raw_part = torch.empty((splits * K * P,), dtype=torch.float32, device=dev)
+            plan = torch.empty(((L.smoe_point_plan_bytes(K, n) + 3) // 4,), dtype=torch.int32, device=dev)
+            check(L.smoe_point_gn_diag(C.byref(self._cfg), ptr(packed), ptr(theta), ptr(indices), ptr(counts), K, n,
+                                       ptr(gstate), ptr(tile_box), splits, ptr(raw_part), ptr(plan), st),
+                  "smoe_point_gn_diag")
+            diag = gn_finalize(self._cfg, raw_part, splits, plan, indices, counts, K, P)
+        return out, dict(zip(PARAM_KEYS, split_grads(diag, self.d, self.C)))
 
     def _check(self, params, points):
         """ValueError for anything __call__ and jacobian cannot take; returns the six parameter tensors."""
